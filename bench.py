@@ -4,9 +4,10 @@
   python bench.py --gpus N --steps K --warmup W                 the B200 path (one process per GPU under torchrun)
   python bench.py --impl reference --gpus N --steps K --warmup W   the reference's own CPU thread-pool path
 
-One JSON line on stdout (rank 0). A "step" is one frame = all views of one scene state. Metric: entities
-transformed+culled+sorted per second (BASELINE.json). `value` is device-resident (SoA already in HBM, lists left in HBM),
-`e2e` goes through the C ABI with host buffers (AoS upload, list download, isVisible write-back) every step.
+One JSON line on stdout (rank 0). A "step" is one frame = all views of one scene state; exactly --steps frames are timed.
+Metric: entities transformed+culled+sorted per second (BASELINE.json). `value` is device-resident (SoA already in HBM, lists
+left in HBM), `e2e` goes through the C ABI with host buffers (AoS upload, list download, isVisible write-back) every step.
+--dump-outputs DIR writes the draw lists of the last timed step (same arguments, same seeded inputs, same files).
 """
 from __future__ import annotations
 
@@ -266,6 +267,57 @@ def stage_scene(sp, scene, views):
     return [m.size for m in pools]
 
 
+DUMP_BYTES = 64 << 20
+RECORD_COLUMNS = 16  # row in the list, componentOffset, bakedModel[12], distanceSq, bufferIndex
+
+
+def dump_outputs(sp, views, out_dir: Path, seed: int):
+    """Writes what a caller of the frame receives (gsp_get_unsorted, gsp_get_sorted, gsp_get_sorted_counts) as float64 .npy
+    files, so that two builds can be compared output for output:
+      counts.npy    one row (view, list, buffer, drawCount, instanceCount) per list of every view: list 0 = unsorted buffer,
+                    1 = translucent list, 2 = UI list (their instanceCount is 0: gsp_get_sorted returns none), 3 = sorted
+                    buffer as gsp_get_sorted_counts reports it
+      view<v>_unsorted<b>.npy, view<v>_translucent.npy, view<v>_ui.npy
+                    rows of RECORD_COLUMNS, one per draw record, in list order; written for the non-empty lists only
+    Every field is exact in float64. Lists that do not fit DUMP_BYTES together are cut to samples of rows (short lists stay
+    whole, the long ones share the rest evenly) whose positions depend only on `seed`, the list's index and the list lengths."""
+    out_dir.mkdir(parents=True, exist_ok=True)
+
+    def fetch(v, which, b):  # (records, drawCount, instanceCount)
+        if which == 0:
+            return sp.get_unsorted(v, b, copy=False)
+        return (*sp.get_sorted(v, which - 1, copy=False), 0)
+
+    lists, counts = [], []
+    for v in range(views.size):
+        lists += [(f"view{v}_unsorted{b}", v, 0, b) for b in range(sp.unsorted_buffer_count(v))]
+        lists += [(f"view{v}_translucent", v, 1, 0), (f"view{v}_ui", v, 2, 0)]
+    for _, v, which, b in lists:
+        counts.append((v, which, b, *fetch(v, which, b)[1:]))
+    counts += [(v, 3, b, *sp.get_sorted_counts(v, b)) for v in range(views.size) for b in range(sp.sorted_buffer_count(v))]
+    np.save(out_dir / "counts.npy", np.array(counts, np.float64))
+    sizes = [c[3] for c in counts[:len(lists)]]
+    caps, left = [0] * len(lists), (DUMP_BYTES - (1 << 20)) // (8 * RECORD_COLUMNS)
+    for k, i in enumerate(sorted(range(len(lists)), key=lambda i: sizes[i])):
+        caps[i] = min(sizes[i], left // (len(lists) - k))
+        left -= caps[i]
+    for i, (name, v, which, b) in enumerate(lists):
+        rec = fetch(v, which, b)[0]
+        if rec.size == 0:
+            continue
+        rows = np.arange(rec.size)
+        if rec.size > caps[i]:
+            rows = np.sort(np.random.default_rng([seed, i]).choice(rec.size, caps[i], replace=False))
+        sel = rec[rows]
+        out = np.empty((rows.size, RECORD_COLUMNS), np.float64)
+        out[:, 0] = rows
+        out[:, 1] = sel["componentOffset"]
+        out[:, 2:14] = sel["bakedModel"]
+        out[:, 14] = sel["distanceSq"]
+        out[:, 15] = sel["bufferIndex"]
+        np.save(out_dir / f"{name}.npy", out)
+
+
 def verify_exchange(workload: str, rank: int, world: int, local_rank: int, stream, per_rank: int = 180_000):
     """Merged-order check over the REAL exchange (NCCL inside the library): a reduced scene of world x per_rank entities is
     cut into contiguous ranges, every rank prepares its range and exchanges, rank 0 also sorts the WHOLE scene on its own GPU;
@@ -363,16 +415,7 @@ def strong_scaling_point(args, rank: int, world: int, local_rank: int, stream):
         pm.frame()
     pm.finish()
     sp.sync()
-    p0, p1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    p0.record(stream)
-    for _ in range(5):
-        pm.frame()
-    p1.record(stream)
-    pm.finish(); sp.sync()
-    reps = max(1, int(np.ceil(args.min_seconds * 0.5e3 / (max(p0.elapsed_time(p1) / 5, 1e-3) * args.steps))))
-    r = torch.tensor([reps], dtype=torch.int64, device="cuda")
-    dist.all_reduce(r, op=dist.ReduceOp.MAX)
-    frames = args.steps * int(r.item())
+    frames = args.steps
     dist.barrier(); torch.cuda.synchronize()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record(stream)
@@ -470,23 +513,7 @@ def run_b200_arm(args):
     if rank == 0:
         sampler.start()
         sampler.wait_first_sample()
-    # a frame lasts well under a millisecond: every step is repeated `reps` times back to back so that the timed region lasts
-    # at least --min-seconds (clocks and power are then sampled under sustained load); ms_per_step stays per FRAME
-    p0, p1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    p0.record(stream)
-    for _ in range(5):
-        frame()
-    p1.record(stream)
-    if merger is not None:
-        merger.finish()
-    sp.sync()
-    probe_ms = max(p0.elapsed_time(p1) / 5, 1e-3)
-    reps = max(1, int(np.ceil(args.min_seconds * 1e3 / (probe_ms * args.steps))))
-    if world > 1:
-        r = torch.tensor([reps], dtype=torch.int64, device="cuda")
-        dist.all_reduce(r, op=dist.ReduceOp.MAX)
-        reps = int(r.item())
-    frames_timed = args.steps * reps
+    frames_timed = args.steps
     ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     barrier()
     t_begin = time.time()
@@ -500,6 +527,8 @@ def run_b200_arm(args):
     barrier()
     t_end = time.time()
     elapsed_ms = ev0.elapsed_time(ev1)
+    if args.dump_outputs:
+        dump_outputs(sp, views, Path(args.dump_outputs), args.seed)
     # latency of ONE frame with nothing overlapped (cull + sort + emit + export + all-gather + merge, serialised)
     latency_ms = None
     exchange_bytes = 0
@@ -766,8 +795,7 @@ def run_b200_arm(args):
             "dtype": "f32", "data": "synthetic",
             "config": {"workload": f"{args.workload}: {desc}", "entities_per_gpu": n, "entities_total": total_entities,
                        "frames_timed": frames_timed,
-                       "timing": f"every one of the {args.steps} steps repeated {reps}x back to back (sustained load, "
-                                 f">= {args.min_seconds} s); ms_per_step is per frame",
+                       "timing": f"{args.steps} frames back to back between two CUDA events; ms_per_step is their mean",
                        "views": int(views.size), "visible_total": int(visible_sum), "shadow_distance": SHADOW_DISTANCE,
                        "l2": "inputs larger than L2 (%.2f GB of SoA streams per frame vs 126 MB L2)" % (75 * n / 1e9),
                        "sharding": ("contiguous entity ranges per GPU, all views per GPU; sorted runs exchanged over NCCL by "
@@ -836,8 +864,6 @@ def main():
     ap.add_argument("--e2e-steps", type=int, default=10)
     ap.add_argument("--ref-sample", type=int, default=0, help="entities the CPU reference runs on (0 = the whole workload)")
     ap.add_argument("--ref-steps", type=int, default=5, help="frames of the in-line cpu_baseline leg")
-    ap.add_argument("--min-seconds", type=float, default=1.0,
-                    help="the device-resident loop repeats every step until the timed region lasts at least this long")
     ap.add_argument("--scaling", default="both", choices=["weak", "strong", "both"],
                     help="N > 1: weak = the workload's N per GPU, strong = the workload's N in total; both = weak is the "
                          "headline value and the strong-scaling numbers go under config.strong")
@@ -847,7 +873,14 @@ def main():
     ap.add_argument("--shadow-distance", type=float, default=0.0,
                     help="CSM shadow distance of the camera + cascades workloads (default 100: the reference's); larger values "
                          "let every cascade see 10-15 %% of the scene (SURVEY.md 8d)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write the draw lists of the last one to DIR/<name>.npy (see dump_outputs); "
+                         "one GPU only: the merged lists of the multi-GPU path are not written")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or int(os.environ.get("WORLD_SIZE", "1")) != 1):
+        ap.error("--dump-outputs writes the lists of the single-GPU B200 path: use it with --impl b200 on one GPU")
     if args.shadow_distance > 0:
         SHADOW_DISTANCE = args.shadow_distance
     if args.impl == "reference":

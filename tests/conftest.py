@@ -11,7 +11,7 @@ for p in (str(ROOT), str(ROOT / "tests")):
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
-    config.addinivalue_line("markers", "multigpu: needs at least two CUDA devices (run with -m multigpu under gpurun --gpus 2)")
+    config.addinivalue_line("markers", "multigpu: needs at least two CUDA devices (skipped where fewer exist)")
 
 
 def _device_usable() -> bool:
@@ -41,14 +41,14 @@ def _gpu_count() -> int:
 
 
 def pytest_collection_modifyitems(config, items):
-    """(1) `multigpu` tests are DESELECTED (not skipped) where fewer than two GPUs exist, so the single-GPU run of `-m gpu`
-    carries no skips. (2) A plain `pytest tests` on a box without a usable sm_100 device skips the gpu-marked tests instead
-    of failing them (tests/test_abi.py::test_no_cpu_fallback stays the one place that asserts the loud failure). With
-    `-m gpu` — how the GPU box runs them — nothing is skipped: a missing device must fail there, not pass silently."""
+    """(1) `multigpu` tests are skipped where fewer than two GPUs exist: they stay in the report of a single-GPU run. (2) A
+    plain `pytest tests` on a box without a usable sm_100 device skips the gpu-marked tests instead of failing them
+    (tests/test_abi.py::test_no_cpu_fallback stays the one place that asserts the loud failure). With `-m gpu` nothing else
+    is skipped: a missing device must fail there, not pass silently."""
     multi = [it for it in items if it.get_closest_marker("multigpu")]
     if multi and _gpu_count() < 2:
-        config.hook.pytest_deselected(items=multi)
-        items[:] = [it for it in items if not it.get_closest_marker("multigpu")]
+        for it in multi:
+            it.add_marker(pytest.mark.skip(reason="needs at least two CUDA devices"))
     markexpr = config.getoption("-m", default="") or ""
     if "gpu" in markexpr and "not gpu" not in markexpr:
         return

@@ -1,6 +1,6 @@
 """The multi-GPU path driven purely through the C ABI by a C++ program (tests/native/exchange_two_ranks.cpp): two GPUs, one
 process, one thread per GPU, NCCL inside the library, no Python in the data path. Needs two devices: marked `multigpu`, which
-tests/conftest.py DESELECTS on a box with fewer than two GPUs (the builder runs it under `gpurun --gpus 2`; log under profiles/)."""
+tests/conftest.py skips on a box with fewer than two GPUs (log of a two-GPU run under profiles/)."""
 import os
 import shutil
 import subprocess
@@ -8,7 +8,7 @@ from pathlib import Path
 
 import pytest
 
-pytestmark = [pytest.mark.gpu, pytest.mark.multigpu]  # (tests/conftest.py deselects `multigpu` items on boxes with fewer than two GPUs)
+pytestmark = [pytest.mark.gpu, pytest.mark.multigpu]
 ROOT = Path(__file__).resolve().parent.parent
 
 

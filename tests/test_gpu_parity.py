@@ -1,4 +1,6 @@
 """GPU parity: the CUDA path (through the C ABI) against the CPU oracle, bit for bit, on seeded scenes."""
+from pathlib import Path
+
 import numpy as np
 import pytest
 
@@ -233,15 +235,63 @@ def test_empty_inputs(sceneprep_lib):
 
 
 # ---- full BASELINE sizes: EVERY list of EVERY view against the reference build ----------------------------------------
-@pytest.mark.parametrize("workload,n", [("C2", 1_000_000), ("C3", 4_000_000), ("C4", 16_000_000)])
+FULL_SIZE = [("C2", 1_000_000), ("C3", 4_000_000), ("C4", 16_000_000)]
+FULL_SIZE_SAMPLES = Path(__file__).resolve().parent / "golden" / "full_size" / "samples.npz"
+SAMPLE_ROWS = 128
+
+
+def _full_size_inputs(scene):
+    """(transform bytes, stride, occupancy, [(pool bytes, stride, occupancy, count)]) of scenes.build_aos(scene)."""
+    tt, pp = scenes.build_aos(scene)
+    pools = [(m.view(np.uint8).reshape(m.size, m.dtype.itemsize), m.dtype.itemsize, m.size, m.size) for m in pp]
+    return tt.view(np.uint8).reshape(tt.size, 80), 80, tt.size, pools
+
+
+def full_size_sample(frames, workload: str) -> dict:
+    """A fixed sample of OracleRun-shaped results: per list its counts, and the raw 64 bytes (key bits, slot, bakedModel
+    bits, buffer index) of SAMPLE_ROWS seeded row positions, which pin the draw order there."""
+    out = {}
+    for v, f in enumerate(frames):
+        lists = [(f"unsorted{b}", rec, draw, inst) for b, (rec, draw, inst) in enumerate(f["unsorted"])]
+        lists += [("trans", *f["trans"], 0), ("ui", *f["ui"], 0)]
+        out[f"{workload}_v{v}_sorted_counts"] = np.array(f["sorted_counts"], np.int64).reshape(-1, 2)
+        for i, (name, rec, draw, inst) in enumerate(lists):
+            rows = np.arange(draw)
+            if draw > SAMPLE_ROWS:
+                rows = np.sort(np.random.default_rng([v, i]).choice(draw, SAMPLE_ROWS, replace=False))
+            out[f"{workload}_v{v}_{name}_counts"] = np.array([draw, inst], np.int64)
+            out[f"{workload}_v{v}_{name}_rows"] = rows.astype(np.int64)
+            out[f"{workload}_v{v}_{name}_records"] = np.ascontiguousarray(rec[:draw][rows]).view(np.uint8).reshape(-1, 64)
+    return out
+
+
+def make_full_size_samples():
+    """Writes FULL_SIZE_SAMPLES from the oracle's results on the inputs test_full_size_vs_reference uses without oracle/_ref
+    (CPU only, a few minutes): `PYTHONPATH=.:tests python -c "import test_gpu_parity as t; t.make_full_size_samples()"`."""
+    import bench
+    out = {}
+    for workload, n in FULL_SIZE:
+        scene = scenes.config_scene(workload, n=n)
+        scene.camera_pos = bench.camera_pos()
+        views = bench.frame_views(workload)
+        t, tstride, tocc, pools = _full_size_inputs(scene)
+        rts = [p.render_type for p in scene.pools]
+        frames = OracleRun((t, tstride, tocc), [(p[0], p[1], p[2]) for p in pools], rts, views, scene.camera_pos).views
+        out.update(full_size_sample(frames, workload))
+    np.savez_compressed(FULL_SIZE_SAMPLES, **out)
+    print(f"{FULL_SIZE_SAMPLES}: {FULL_SIZE_SAMPLES.stat().st_size / 1024:.0f} KiB")
+
+
+@pytest.mark.parametrize("workload,n", FULL_SIZE)
 def test_full_size_vs_reference(sceneprep_lib, oracle_built, workload, n):
     """At BASELINE.json's sizes: the scene is built through the reference's real ECS (oracle/_ref parity build: the
     reference's own mesh.cpp / transform.cpp, SURVEY.md 8c), the CUDA path consumes the raw bytes of the reference's live
     pools, and every draw list of every view is compared with the reference's — key bits, draw order (the reference's
     order canonicalised inside equal-key runs, ours must already be canonical), bakedModel bits, counts — plus isVisible of
-    every slot. A wrongly culled entity anywhere in the scene fails this test. Without oracle/_ref (never the case on the
-    GPU box: it travels with the snapshot) the pinned C oracle takes the reference's place. Then idempotence: a second
-    frame over the same state gives identical lists."""
+    every slot. A wrongly culled entity anywhere in the scene fails this test. Without oracle/_ref (a clean checkout) the
+    pinned C oracle takes the reference's place, and a stored sample of the lists (tests/golden/full_size/samples.npz, see
+    full_size_sample) must match as well, so that a change made alike to the oracle and the CUDA path is still caught. Then
+    idempotence: a second frame over the same state gives identical lists."""
     import bench
     import reflib
     from common import assert_frames_equal, gpu_frame, ref_frame
@@ -263,11 +313,13 @@ def test_full_size_vs_reference(sceneprep_lib, oracle_built, workload, n):
         ref.close()
         canonicalise_want = True
     else:
-        tt, pp = scenes.build_aos(scene)
-        t, tstride, tocc = tt.view(np.uint8).reshape(tt.size, 80), 80, tt.size
-        pools = [(m.view(np.uint8).reshape(m.size, m.dtype.itemsize), m.dtype.itemsize, m.size, m.size) for m in pp]
-        orun = OracleRun((t, tstride, tocc), [(p[0], p[1], p[2]) for p in pools], rts, views, scene.camera_pos)
-        want = orun.views
+        t, tstride, tocc, pools = _full_size_inputs(scene)
+        want = OracleRun((t, tstride, tocc), [(p[0], p[1], p[2]) for p in pools], rts, views, scene.camera_pos).views
+        stored = np.load(FULL_SIZE_SAMPLES)
+        got_sample = full_size_sample(want, workload)
+        assert sorted(got_sample) == sorted(k for k in stored.files if k.startswith(workload + "_"))
+        for k, a in got_sample.items():
+            assert np.array_equal(a, stored[k]), f"{workload} {n}: {k} differs from the stored sample"
     del scene
     sp = ScenePrep(0)
     sp.set_transforms(t, tstride, tocc)

@@ -28,5 +28,5 @@ timeout 400 python bench.py --shadow-distance 1200 --no-cpu-baseline > $O/r2_ben
 
 # 4. launch list of the default command (per-launch times are cold-cache and serialised: shares, not absolutes)
 timeout 600 ncu --metrics gpu__time_duration.sum --clock-control none -c 400 --csv --log-file $O/r2_launches_c4_16M.csv \
-    python bench.py --steps 2 --warmup 1 --no-cpu-baseline --min-seconds 0 --e2e-steps 1 > $O/bench_under_ncu.log 2>&1
+    python bench.py --steps 2 --warmup 1 --no-cpu-baseline --e2e-steps 1 > $O/bench_under_ncu.log 2>&1
 tail -2 $O/r2_gpu_tests.log; cat $O/r2_smoke.log | tail -1; head -c 600 $O/r2_bench_c4_16M.json; echo; head -c 300 $O/r2_bench_reference_c4_16M.json

@@ -11,5 +11,5 @@ timeout 300 python bench.py --workload C2 --no-cpu-baseline > $O/r2_bench_c2_1M.
 timeout 300 python bench.py --workload C5 --no-cpu-baseline > $O/r2_bench_c5_shard_8M_16views_1gpu.json 2> $O/bench_c5.err
 timeout 300 python bench.py --shadow-distance 600 --no-cpu-baseline > $O/r2_bench_c4_16M_shadow600.json 2> $O/bench_s600.err
 timeout 300 python bench.py --shadow-distance 1200 --no-cpu-baseline > $O/r2_bench_c4_16M_shadow1200.json 2> $O/bench_s1200.err
-timeout 300 ncu --metrics gpu__time_duration.sum --clock-control none -c 400 --csv --log-file $O/r2_launches_c4_16M.csv python bench.py --steps 2 --warmup 1 --no-cpu-baseline --min-seconds 0 --e2e-steps 1 > $O/bench_under_ncu.log 2>&1
+timeout 300 ncu --metrics gpu__time_duration.sum --clock-control none -c 400 --csv --log-file $O/r2_launches_c4_16M.csv python bench.py --steps 2 --warmup 1 --no-cpu-baseline --e2e-steps 1 > $O/bench_under_ncu.log 2>&1
 tail -2 $O/r2_gpu_tests.log; tail -1 $O/r2_smoke.log; head -c 330 $O/r2_bench_c4_16M.json
