@@ -274,6 +274,7 @@ int gsp_set_transforms(gsp_context* ctx, const void* aos, uint32_t stride, uint3
 		t.capacity = cap;
 	}
 	t.occupancy = occupancy;
+	t.cyclic = false;
 	c.linkDirty = true; c.chainDirty = true; c.resultsValid = false; c.frameEnqueued = false;
 	if (occupancy == 0)
 		return GSP_OK;
@@ -292,12 +293,25 @@ int gsp_set_transforms(gsp_context* ctx, const void* aos, uint32_t stride, uint3
 	// entity -> slot map sized by the largest live entity id, then parent slots and chain lengths from the SoA copy
 	GSP_CUDA(ensureDevice32(t.entityToSlot, t.entityCap, (size_t)maxEntity + 1));
 	GSP_CUDA(cudaMemsetAsync(t.entityToSlot, 0, (size_t)t.entityCap * sizeof(uint32_t), c.stream));
-	launchBuildHierarchy(c);
-	GSP_CUDA(cudaMemcpyAsync(&hScalars[1], c.dError, sizeof(uint32_t), cudaMemcpyDeviceToHost, c.stream));
+	uint32_t* dFlag = dMax; // (read already) set when some chain is 255 links or longer, then when some chain is cyclic
+	GSP_CUDA(cudaMemsetAsync(dFlag, 0, sizeof(uint32_t), c.stream));
+	launchBuildHierarchy(c, dFlag);
+	GSP_CUDA(cudaMemcpyAsync(&hScalars[1], c.dError, 2 * sizeof(uint32_t), cudaMemcpyDeviceToHost, c.stream)); // error, flag
 	GSP_CUDA(cudaStreamSynchronize(c.stream));
 	GSP_CUDA(cudaGetLastError());
 	if (hScalars[1])
 		return fail(c, GSP_ERR_HIERARCHY, "gsp_set_transforms: a parent entity has no TransformComponent");
+	if (hScalars[2])
+	{
+		// deep chains are legal; cycles are recorded here and refused by every call that walks the chains (gsp_run,
+		// gsp_set_active, gsp_animate), so those walks need no per-frame cycle guard
+		GSP_CUDA(cudaMemsetAsync(dFlag, 0, sizeof(uint32_t), c.stream));
+		launchFindCycles(c, dFlag);
+		GSP_CUDA(cudaMemcpyAsync(&hScalars[2], dFlag, sizeof(uint32_t), cudaMemcpyDeviceToHost, c.stream));
+		GSP_CUDA(cudaStreamSynchronize(c.stream));
+		GSP_CUDA(cudaGetLastError());
+		t.cyclic = hScalars[2] != 0;
+	}
 	return GSP_OK;
 }
 
@@ -708,6 +722,8 @@ int gsp_run_async(gsp_context* ctx)
 	Context& c = ctx->c;
 	if (!c.viewsSet)
 		return fail(c, GSP_ERR_STATE, "gsp_run: gsp_set_views has not been called");
+	if (c.tf.cyclic)
+		return fail(c, GSP_ERR_HIERARCHY, "gsp_run: the transform hierarchy is cyclic");
 	GSP_CUDA(cudaSetDevice(c.device));
 	c.fetchedValid = false; // the record arena and the counters are about to be rewritten
 	if (c.fetchInFlight) // the previous frame's lists are still travelling out of the record arena
@@ -783,7 +799,7 @@ int gsp_sync(gsp_context* ctx)
 	if (!c.frameEnqueued || c.layoutDirty)
 		return fail(c, GSP_ERR_STATE, "gsp_sync: no frame has been enqueued (gsp_run_async) since the last change");
 	if (c.hCounters[kCtrError])
-		return fail(c, GSP_ERR_HIERARCHY, "gsp_run: transform hierarchy is cyclic or deeper than 4096");
+		return fail(c, GSP_ERR_HIERARCHY, "gsp_run: a parent chain is longer than the transform pool");
 	c.resultsValid = true;
 	return GSP_OK;
 }
@@ -1171,6 +1187,8 @@ int gsp_set_active(gsp_context* ctx, const uint32_t* entityIds, uint32_t count, 
 	auto& t = c.tf;
 	if (!t.flags || !t.entityToSlot)
 		return fail(c, GSP_ERR_STATE, "gsp_set_active: gsp_set_transforms has not been called");
+	if (t.cyclic)
+		return fail(c, GSP_ERR_HIERARCHY, "gsp_set_active: the transform hierarchy is cyclic (nothing was applied)");
 	GSP_CUDA(cudaSetDevice(c.device));
 	uint32_t* dIds = nullptr;
 	if (count)
@@ -1191,7 +1209,7 @@ int gsp_set_active(gsp_context* ctx, const uint32_t* entityIds, uint32_t count, 
 	GSP_CUDA(cudaGetLastError());
 	c.resultsValid = false; c.frameEnqueued = false;
 	if (hScalars[1] == (uint32_t)GSP_ERR_HIERARCHY)
-		return fail(c, GSP_ERR_HIERARCHY, "gsp_set_active: transform hierarchy is cyclic or deeper than 4096");
+		return fail(c, GSP_ERR_HIERARCHY, "gsp_set_active: a parent chain is longer than the transform pool");
 	if (hScalars[1])
 		return fail(c, GSP_ERR_INVALID, "gsp_set_active: an entity id has no TransformComponent (the other ids were applied)");
 	return GSP_OK;
@@ -1209,6 +1227,8 @@ int gsp_animate(gsp_context* ctx, const uint32_t* entityIds, const uint8_t* flag
 		return fail(c, GSP_ERR_STATE, "gsp_animate: gsp_set_transforms has not been called");
 	if (count == 0)
 		return GSP_OK;
+	if (tf.cyclic)
+		return fail(c, GSP_ERR_HIERARCHY, "gsp_animate: the transform hierarchy is cyclic (nothing was animated)");
 	GSP_CUDA(cudaSetDevice(c.device));
 	// one upload: ids | t | frameA | frameB | flags
 	const size_t idBytes = (size_t)count * 4, frameBytes = (size_t)count * 40, flagBytes = ((size_t)count + 15) & ~(size_t)15;
@@ -1238,7 +1258,7 @@ int gsp_animate(gsp_context* ctx, const uint32_t* entityIds, const uint8_t* flag
 	GSP_CUDA(cudaGetLastError());
 	c.chainDirty = true; c.resultsValid = false; c.frameEnqueued = false;
 	if (hScalars[1] == (uint32_t)GSP_ERR_HIERARCHY)
-		return fail(c, GSP_ERR_HIERARCHY, "gsp_animate: transform hierarchy is cyclic or deeper than 4096");
+		return fail(c, GSP_ERR_HIERARCHY, "gsp_animate: a parent chain is longer than the transform pool");
 	if (hScalars[1])
 		return fail(c, GSP_ERR_INVALID, "gsp_animate: an entity id has no TransformComponent (the other entities were animated)");
 	return GSP_OK;

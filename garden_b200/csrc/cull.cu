@@ -59,6 +59,7 @@ struct CullArgs
 	const uint32_t* __restrict__ tIndex;  // transform slot -> index in tList (only meaningful where tList[index] == slot)
 	float4* __restrict__ tWorld;          // [surviving transform][kWorldStride] chain product, camera NOT subtracted
 	uint32_t tCounter;                    // counter index holding the length of tList
+	uint32_t tOccupancy;                  // transform slots: no acyclic chain has more links
 };
 
 constexpr uint32_t kChunkTiles = 8;                                // 256-survivor tiles per compaction chunk
@@ -584,7 +585,7 @@ static __device__ __forceinline__ void walkChainSlow(const CullShared& sh, const
 	uint32_t depth = 0;
 	while (p != kNone)
 	{
-		if (++depth > kMaxChainDepth)
+		if (++depth > a.tOccupancy) // (cannot happen: cyclic hierarchies are refused before launch)
 		{
 			atomicExch(&a.counters[kCtrError], (uint32_t)GSP_ERR_HIERARCHY);
 			break;
@@ -1060,7 +1061,7 @@ static __device__ __noinline__ Mat43 chainFromStreams(const CullArgs& a, uint32_
 	uint32_t p = a.tParent[ts], depth = 0;
 	while (p != kNone)
 	{
-		if (++depth > kMaxChainDepth)
+		if (++depth > a.tOccupancy) // (cannot happen: cyclic hierarchies are refused before launch)
 		{
 			atomicExch(&a.counters[kCtrError], (uint32_t)GSP_ERR_HIERARCHY);
 			break;
@@ -1497,6 +1498,7 @@ static void commonArgs(Context& c, CullArgs& A)
 {
 	A.tRot = c.tf.rot; A.tPosSx = c.tf.posSx; A.tSYZ = c.tf.sYZ; A.tParent = c.tf.parent; A.tFlags = c.tf.flags;
 	A.tRecord = c.tf.record;
+	A.tOccupancy = c.tf.occupancy;
 	A.counters = c.dCounters;
 	A.tList = c.tf.tList; A.tIndex = c.tf.tIndex; A.tWorld = c.tf.tWorld; A.tCounter = kCtrSurvivorsT;
 	static const bool prepassOff = []{ const char* e = getenv("GSP_PREPASS"); return e && !strcmp(e, "0"); }();

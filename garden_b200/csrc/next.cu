@@ -95,7 +95,7 @@ __global__ void __launch_bounds__(256) kPropagateActive(uint32_t count, const ui
 	uint32_t p = parent[i], depth = 0;
 	while (p != kNone && anc)
 	{
-		if (++depth > kMaxChainDepth)
+		if (++depth > count) // (cannot happen: cyclic hierarchies are refused before launch)
 		{
 			atomicExch(error, (uint32_t)GSP_ERR_HIERARCHY);
 			break;

@@ -13,7 +13,6 @@ namespace gsp
 constexpr uint32_t kNone = 0xFFFFFFFFu;
 constexpr int kMaxPools = GSP_MAX_POOLS;
 constexpr int kMaxViews = GSP_MAX_VIEWS;
-constexpr uint32_t kMaxChainDepth = 4096; // guard against cyclic hierarchies
 
 // ---- AoS field offsets of the reference's components (SURVEY.md §8 a1/a2, verified with offsetof in oracle/ref_harness) ----
 // TransformComponent, include/garden/system/transform.hpp:31-60
@@ -66,6 +65,10 @@ struct TransformsDev
 	uint32_t splitCap = 0;
 	uint32_t* entityToSlot = nullptr; // entity id -> slot + 1
 	uint32_t entityCap = 0;
+	// some parent chain is cyclic (decided once per gsp_set_transforms, staging.cu: kJumpParents): nothing walks the chains
+	// then, so an acyclic hierarchy of any depth is walked to its roots and the per-frame walks only keep `occupancy` as a
+	// bound against corrupted links
+	bool cyclic = false;
 };
 
 struct PoolDev
@@ -250,7 +253,8 @@ constexpr uint32_t kExMagic = 0x47535031u; // "GSP1"
 // ---- kernel launchers (each returns the number of kernels it launched, or throws nothing; errors via cudaGetLastError) ----
 uint32_t launchStageTransforms(Context& c, const void* dAos, uint32_t stride, uint32_t first, uint32_t count, bool full,
 	uint32_t* dMaxEntity, const uint32_t* dSlotMap = nullptr);
-uint32_t launchBuildHierarchy(Context& c);
+uint32_t launchBuildHierarchy(Context& c, uint32_t* dDeep);
+uint32_t launchFindCycles(Context& c, uint32_t* dCyclic);
 uint32_t launchStagePool(Context& c, uint32_t pool, const void* dAos, uint32_t stride, uint32_t occupancy);
 uint32_t launchLink(Context& c);
 uint32_t launchChainBounds(Context& c);

@@ -147,8 +147,9 @@ __global__ void __launch_bounds__(256) kResolveParents(uint32_t count, const uin
 
 // Chain length of every transform (number of ancestors, saturating at 255) into the upper flag byte. The cull kernel uses
 // it as the trip count of its chain loop and to group work of equal chain length into the same warp; a wrong value only
-// costs time (the links decide), never correctness.
-__global__ void __launch_bounds__(256) kComputeDepth(uint32_t count, const uint32_t* __restrict__ parent, uint16_t* __restrict__ flags)
+// costs time (the links decide), never correctness. *deep = 1 when some walk saturates: only then can a chain be cyclic.
+__global__ void __launch_bounds__(256) kComputeDepth(uint32_t count, const uint32_t* __restrict__ parent, uint16_t* __restrict__ flags,
+	uint32_t* __restrict__ deep)
 {
 	uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
 	if (i >= count)
@@ -160,7 +161,27 @@ __global__ void __launch_bounds__(256) kComputeDepth(uint32_t count, const uint3
 		depth++;
 		p = parent[p];
 	}
+	if (depth == kTfDepthMax)
+		*deep = 1;
 	flags[i] = (uint16_t)((flags[i] & ((1u << kTfDepthShift) - 1u)) | (depth << kTfDepthShift));
+}
+
+// Cycle detection by pointer jumping. up[i] starts as the parent link; every round replaces it by the link of the slot it
+// points at, so after r rounds it points at least 2^r steps up the chain, or is kNone past the root. A round may read a link
+// that another thread of the same round has already advanced: that only moves further up the same chain. An acyclic chain has
+// at most count - 1 links, so after ceil(log2(count)) rounds every link still set lies on a cycle or leads into one.
+__global__ void __launch_bounds__(256) kJumpParents(uint32_t count, uint32_t* up, uint32_t* __restrict__ cyclic)
+{
+	uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+	if (i >= count)
+		return;
+	uint32_t p = up[i];
+	if (p == kNone)
+		return;
+	p = up[p];
+	up[i] = p;
+	if (cyclic && p != kNone)
+		*cyclic = 1;
 }
 
 // One block per tile of mesh-component slots: AABB, owner entity, the static part of the filter at mesh.cpp:140-147, and the
@@ -263,8 +284,9 @@ uint32_t launchStageTransforms(Context& c, const void* dAos, uint32_t stride, ui
 	return 1;
 }
 
-// After a full staging pass: entity map, parent slots, chain lengths (all from the SoA copy in HBM).
-uint32_t launchBuildHierarchy(Context& c)
+// After a full staging pass: entity map, parent slots, chain lengths (all from the SoA copy in HBM). *dDeep (zeroed by the
+// caller) is set when some chain is 255 links or longer.
+uint32_t launchBuildHierarchy(Context& c, uint32_t* dDeep)
 {
 	auto& t = c.tf;
 	const uint32_t count = t.occupancy;
@@ -273,8 +295,25 @@ uint32_t launchBuildHierarchy(Context& c)
 	kBuildEntityMap<<<blocksFor(count, 256), 256, 0, c.stream>>>(count, t.entity, t.entityToSlot);
 	kResolveParents<<<blocksFor(count, 256), 256, 0, c.stream>>>(count, t.parentEntity, t.entityToSlot, t.entityCap,
 		t.parent, c.dError);
-	kComputeDepth<<<blocksFor(count, 256), 256, 0, c.stream>>>(count, t.parent, t.flags);
+	kComputeDepth<<<blocksFor(count, 256), 256, 0, c.stream>>>(count, t.parent, t.flags, dDeep);
 	return 3;
+}
+
+// *dCyclic (zeroed by the caller) = 1 iff some parent chain is cyclic. Only run when launchBuildHierarchy found a deep chain.
+// The jump links live in chainRoot, which gsp_set_transforms marks stale (kChainBounds rewrites it before it is read).
+uint32_t launchFindCycles(Context& c, uint32_t* dCyclic)
+{
+	auto& t = c.tf;
+	const uint32_t count = t.occupancy;
+	if (count == 0)
+		return 0;
+	uint32_t rounds = 1;
+	while ((1ull << rounds) < count)
+		rounds++;
+	cudaMemcpyAsync(t.chainRoot, t.parent, (size_t)count * sizeof(uint32_t), cudaMemcpyDeviceToDevice, c.stream);
+	for (uint32_t r = 0; r < rounds; r++)
+		kJumpParents<<<blocksFor(count, 256), 256, 0, c.stream>>>(count, t.chainRoot, r + 1 == rounds ? dCyclic : nullptr);
+	return rounds;
 }
 
 uint32_t launchStagePool(Context& c, uint32_t pool, const void* dAos, uint32_t stride, uint32_t occupancy)

@@ -32,8 +32,9 @@ typedef enum gsp_status
 	GSP_ERR_CUDA = 2,     /* CUDA runtime / device error (see gsp_last_error) */
 	GSP_ERR_NOMEM = 3,    /* host or device allocation failed */
 	GSP_ERR_STATE = 4,    /* call sequence error (e.g. gsp_run before gsp_set_views) */
-	GSP_ERR_HIERARCHY = 5 /* a parent entity has no TransformComponent or the chain is cyclic
-	                         (the reference throws EcsmError from Manager::get, ecsm.hpp:863-873) */
+	GSP_ERR_HIERARCHY = 5 /* a parent entity has no TransformComponent (gsp_set_transforms; the reference throws EcsmError
+	                         from Manager::get, ecsm.hpp:863-873), or the hierarchy is cyclic (gsp_run, gsp_set_active,
+	                         gsp_animate). Acyclic chains of any depth are valid. */
 } gsp_status;
 
 /* MeshRenderType — include/garden/system/render/mesh.hpp:30-40 (same numeric values). */

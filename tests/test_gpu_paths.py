@@ -12,7 +12,7 @@ import pytest
 pytestmark = pytest.mark.gpu
 ROOT = Path(__file__).resolve().parent.parent
 QUICK = ["tests/test_gpu_fuzz.py", "tests/test_gpu_golden.py", "tests/test_gpu_next.py", "tests/test_gpu_hostpath.py",
-         "tests/test_gpu_parity.py"]
+         "tests/test_gpu_parity.py", "tests/test_gpu_shapes.py"]
 
 
 @pytest.mark.parametrize("env", [{"GSP_SPLIT": "1"}, {"GSP_SPLIT": "0"}, {"GSP_PREPASS": "0"}, {"GSP_BOXGROUP": "0"},
