@@ -48,11 +48,9 @@ SYMBOLS = {
     "gsp_list_count": (_u32, [_vp]),
     "gsp_get_list_counts": (_i32, [_vp, _vp, _u32]),
     "gsp_export_runs": (_i32, [_vp, _vp, _vp, _u32]),
-    "gsp_merge_gathered": (_i32, [_vp, _u32, _u32, _u32, _u32, _vp, _vp, _vp, _vp, _u32, _vp, _vp, _vp, _vp, _vp, _vp]),
     "gsp_exchange_block_words": (_u32, [_u32]),
     "gsp_merge_plan_words": (_u32, [_u32, _u32]),
     "gsp_export_runs_packed": (_i32, [_vp, _vp, _u32]),
-    "gsp_merge_gathered_packed": (_i32, [_vp, _u32, _u32, _u32, _u32, _vp, _vp, _vp, _vp, _vp, _vp, _u32]),
     "gsp_merge_tree_scratch_words": (_u64, [_u32]),
     "gsp_merge_gathered_packed_tree": (_i32, [_vp, _u32, _u32, _u32, _u32, _vp, _vp, _vp, _vp, _vp, _vp, _u32, _vp]),
     "gsp_comm_unique_id": (_i32, [_vp]),

@@ -182,10 +182,8 @@ int gsp_set_stream(gsp_context* ctx, void* cudaStream)
 //    staging kernel ("zero copy") — no intermediate device buffer, the re-layout overlaps the transfer;
 //  * device memory: read in place;
 //  * pageable host memory: copied into a device scratch buffer first (cudaMemcpyAsync stages it through the driver).
-// GSP_UPLOAD=copy in the environment forces the scratch path for pinned memory too (A/B measurements).
 static int resolveSource(Context& c, const void* aos, size_t bytes, const void** src)
 {
-	static const bool forceCopy = []{ const char* e = getenv("GSP_UPLOAD"); return e && !strcmp(e, "copy"); }();
 	cudaPointerAttributes attr = {};
 	cudaError_t err = cudaPointerGetAttributes(&attr, aos);
 	if (err != cudaSuccess)
@@ -198,7 +196,7 @@ static int resolveSource(Context& c, const void* aos, size_t bytes, const void**
 		*src = attr.devicePointer;
 		return GSP_OK;
 	}
-	if (attr.type == cudaMemoryTypeHost && attr.devicePointer && !forceCopy)
+	if (attr.type == cudaMemoryTypeHost && attr.devicePointer)
 	{
 		*src = attr.devicePointer;
 		c.zeroCopyBytes += bytes;

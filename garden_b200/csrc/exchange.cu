@@ -13,7 +13,7 @@
 //              same weighted quantiles, each rank packs one sub-block per destination, grouped ncclSend/ncclRecv move them,
 //              and a rank receives only what it merges: 1/ranks of the all-gather's volume. Sub-block headers also carry
 //              "elements of the sender's run below your key range", whose sum is where the slice starts in the merged list.
-// The merge is a pairwise merge-path tree (merge.cu: kMergeTree; GSP_MERGE=slice selects round 1's rank-in-every-run merge).
+// Both protocols merge with the same pairwise merge-path tree (merge.cu: kTreePartition + kMergeTree).
 // The block capacity is speculative: an overflow is flagged in the header and in the plan flags, nothing is merged for
 // that frame, and the host — which reads the flags from pinned memory — grows the blocks and repeats the frame.
 #include "sceneprep_internal.h"
@@ -112,7 +112,6 @@ struct Exchange
 	bool allToAll = true, timing = false;
 	uint32_t* dScalar = nullptr; // 2 words for the autosize reduction
 	uint32_t* mergeScratch = nullptr; // the two intermediate levels of the merge tree (merges are serialised on `stream`)
-	bool treeMerge = true;            // GSP_MERGE=slice: rank every element in every other run instead (kMergeSlice)
 };
 
 } // namespace gsp
@@ -203,8 +202,6 @@ static int attachComm(Context& c, ncclComm_t comm, uint32_t ranks, uint32_t rank
 	x->comm = comm; x->ranks = ranks; x->rank = rank;
 	const char* mode = getenv("GSP_EXCHANGE");
 	x->allToAll = !(mode && !strcmp(mode, "allgather"));
-	const char* merge = getenv("GSP_MERGE");
-	x->treeMerge = !(merge && !strcmp(merge, "slice"));
 	c.exchange = x;
 	GSP_CUDA(cudaSetDevice(c.device));
 	GSP_CUDA(cudaStreamCreateWithFlags(&x->stream, cudaStreamNonBlocking));
@@ -234,6 +231,8 @@ static int allocateSets(Context& c, uint32_t capacity)
 	const size_t outCap = (size_t)capacity * ranks;
 	if (outCap > 0xFFFFFFF0ull)
 		return failEx(c, GSP_ERR_NOMEM, "exchange capacity exceeds 2^32 elements");
+	if (!exchangeBlocksIndexable(capacity, ranks))
+		return failEx(c, GSP_ERR_NOMEM, "exchange blocks of all ranks reach 2^32 words (the merge indexes them with 32 bits)");
 	const size_t planWords = 2ull * ranks * lists + lists + 2ull * lists * ranks + 8;
 	for (auto& s : x.sets)
 	{
@@ -251,8 +250,7 @@ static int allocateSets(Context& c, uint32_t capacity)
 		GSP_CUDA(cudaMallocHost((void**)&s.hFlags, 8 * sizeof(uint32_t)));
 		memset(s.hFlags, 0, 8 * sizeof(uint32_t));
 	}
-	if (x.treeMerge)
-		GSP_CUDA(cudaMalloc((void**)&x.mergeScratch, gsp_merge_tree_scratch_words((uint32_t)outCap) * sizeof(uint32_t)));
+	GSP_CUDA(cudaMalloc((void**)&x.mergeScratch, gsp_merge_tree_scratch_words((uint32_t)outCap) * sizeof(uint32_t)));
 	x.capacity = capacity; x.outCapacity = (uint32_t)outCap;
 	return GSP_OK;
 }
@@ -278,7 +276,7 @@ int gsp_comm_init(gsp_context* ctx, const uint8_t id[GSP_COMM_ID_BYTES], uint32_
 	if (!ctx || !id)
 		return GSP_ERR_INVALID;
 	Context& c = ctx->c;
-	if (ranks == 0 || ranks > 32 || rank >= ranks)
+	if (ranks == 0 || ranks > kMaxRanks || rank >= ranks)
 		return failEx(c, GSP_ERR_INVALID, "gsp_comm_init: need 1 <= ranks <= 32 and rank < ranks");
 	NcclApi& N = nccl();
 	if (!N.CommInitRank)
@@ -293,7 +291,7 @@ int gsp_comm_init(gsp_context* ctx, const uint8_t id[GSP_COMM_ID_BYTES], uint32_
 
 int gsp_comm_init_all(gsp_context** contexts, uint32_t count)
 {
-	if (!contexts || count == 0 || count > 32)
+	if (!contexts || count == 0 || count > kMaxRanks)
 		return GSP_ERR_INVALID;
 	for (uint32_t i = 0; i < count; i++)
 		if (!contexts[i]) return GSP_ERR_INVALID;
@@ -301,8 +299,8 @@ int gsp_comm_init_all(gsp_context** contexts, uint32_t count)
 	NcclApi& N = nccl();
 	if (!N.CommInitAll)
 		return failEx(c, GSP_ERR_CUDA, N.error.empty() ? "NCCL is not available" : N.error.c_str());
-	int devices[32];
-	ncclComm_t comms[32];
+	int devices[kMaxRanks];
+	ncclComm_t comms[kMaxRanks];
 	for (uint32_t i = 0; i < count; i++)
 		devices[i] = contexts[i]->c.device;
 	GSP_NCCL(N.CommInitAll(comms, (int)count, devices));

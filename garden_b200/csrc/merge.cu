@@ -1,12 +1,13 @@
-// Multi-GPU exchange step: k-way merge of the per-GPU sorted (key, payload) runs after the NCCL all-gather.
+// Multi-GPU exchange step: k-way merge of the per-GPU sorted (key, payload) runs once they have been exchanged (exchange.cu).
 //
 // The reference has no counterpart (one process, one std::sort per list, mesh.cpp:265-328); this is what makes the sharded
 // path produce the same draw order as a single sort over all entities: every GPU culls + sorts its contiguous entity
-// range, the runs are all-gathered over NVLink, and each GPU merges ONE key range of every list (splitters are taken from
-// the longest run, which every rank holds after the gather, so all ranks agree without further communication).
-// Position of an element = sum over the runs of (number of elements that precede it); ties are broken by (rank, payload),
-// i.e. by global entity order, because shards are contiguous ranges in rank order and runs are already tie-ordered by
-// payload (stable radix sort of a slot-ordered compaction).
+// range, the runs travel over NVLink, and each GPU merges ONE key range of every list. Either the runs were cut by common
+// splitters before they travelled (all-to-all: every received element is mine), or every rank received every run
+// (all-gather) and kMergeBounds cuts my range out of each (splitters are taken from the longest run, which every rank holds,
+// so all ranks agree without further communication). The sub-ranges are then merged two by two by a merge-path tree
+// (kTreePartition + kMergeTree). Ties are broken by (rank, payload), i.e. by global entity order, because shards are
+// contiguous ranges in rank order and runs are already tie-ordered by payload (stable radix sort of a slot-ordered compaction).
 #include "sceneprep_internal.h"
 #include <algorithm>
 
@@ -31,9 +32,7 @@ struct MergeArgs
 
 // Warp-cooperative bound: all 32 lanes call it with the same arguments. Every round probes 32 evenly spaced positions of the
 // remaining range and keeps the 1/33 of it that contains the answer, so a run of millions of keys takes 4-5 dependent
-// memory round trips instead of 22 (the searches that bracket a chunk are pure latency).
-// kUpper: first index with a[i] > key, else first index with a[i] >= key.
-template<bool kUpper>
+// memory round trips instead of 22 (the searches are pure latency). Returns the first index with a[i] >= key.
 __device__ __forceinline__ uint32_t warpBound(const uint32_t* __restrict__ a, uint32_t n, uint32_t key)
 {
 	const uint32_t lane = threadIdx.x & 31;
@@ -43,7 +42,7 @@ __device__ __forceinline__ uint32_t warpBound(const uint32_t* __restrict__ a, ui
 		const uint64_t span = hi - lo;
 		const uint32_t p = lo + (uint32_t)(((uint64_t)(lane + 1) * span) / 33); // lo < p < hi, increasing with the lane
 		const uint32_t v = a[p];
-		const uint32_t before = __ballot_sync(0xffffffffu, kUpper ? v <= key : v < key); // a prefix of the lanes
+		const uint32_t before = __ballot_sync(0xffffffffu, v < key); // a prefix of the lanes
 		const uint32_t t = __popc(before);
 		const uint32_t pPrev = __shfl_sync(0xffffffffu, p, t ? t - 1 : 0), pNext = __shfl_sync(0xffffffffu, p, t < 32 ? t : 31);
 		if (t) lo = pPrev + 1;
@@ -51,7 +50,7 @@ __device__ __forceinline__ uint32_t warpBound(const uint32_t* __restrict__ a, ui
 	}
 	const uint32_t i = lo + lane;
 	const uint32_t v = i < hi ? a[i] : 0u;
-	const uint32_t before = __ballot_sync(0xffffffffu, i < hi && (kUpper ? v <= key : v < key));
+	const uint32_t before = __ballot_sync(0xffffffffu, i < hi && v < key);
 	return lo + __popc(before);
 }
 
@@ -79,8 +78,8 @@ __global__ void __launch_bounds__(1024) kMergeBounds(const __grid_constant__ Mer
 		uint32_t lo = 0u, hi = n;
 		if (!A.preSplit)
 		{
-			lo = hasLo ? warpBound<false>(a, n, keyLo) : 0u;
-			hi = hasHi ? warpBound<false>(a, n, keyHi) : n;
+			lo = hasLo ? warpBound(a, n, keyLo) : 0u;
+			hi = hasHi ? warpBound(a, n, keyHi) : n;
 		}
 		if (hi < lo) hi = lo; // equal splitters
 		if (lane == 0)
@@ -103,139 +102,18 @@ __global__ void __launch_bounds__(1024) kMergeBounds(const __grid_constant__ Mer
 	}
 }
 
-// grid (blocks, ranks, lists): a block takes chunks of kMergeChunk consecutive elements of one run's sub-range and places
-// them into my slice. Positions inside the other runs are monotone along the run, so the block first brackets the chunk in
-// every other run (warp-cooperative searches), then copies the bracketed windows — together about ranks x chunk keys —
-// into shared memory with coalesced loads, and every element ranks itself in every window by a binary search in SHARED
-// memory (a scattered global search costs one L1 wavefront per lane, a shared one roughly one per warp). A chunk whose
-// windows do not fit (very uneven key densities between ranks) searches the brackets in global memory instead.
-constexpr uint32_t kMergeThreads = 256, kMergeChunk = 1024, kMergeWindow = 10240; // window keys staged per chunk (40 KB)
-template<bool kUpper> // kUpper: count elements <= key (ties go to the other run), else elements < key
-__device__ __forceinline__ uint32_t boundIn(const uint32_t* __restrict__ a, uint32_t lo, uint32_t hi, uint32_t key)
-{
-	while (lo < hi)
-	{
-		const uint32_t mid = (lo + hi) >> 1;
-		const uint32_t v = a[mid];
-		if (kUpper ? v <= key : v < key) lo = mid + 1; else hi = mid;
-	}
-	return lo;
-}
-// Brackets a chunk [firstKey, lastKey] of run `run` in every other run: the block's warps share the 2 * (ranks - 1)
-// searches, each done cooperatively by a whole warp. Lower ranks win ties (they hold lower global entity indices), so
-// runs below `run` are searched with the upper bound.
-__device__ __forceinline__ void bracketChunk(const MergeArgs& A, uint32_t list, uint32_t run, uint32_t firstKey, uint32_t lastKey,
-	uint32_t* sLo, uint32_t* sHi)
-{
-	const uint32_t warp = threadIdx.x >> 5, warps = blockDim.x >> 5, lane = threadIdx.x & 31;
-	for (uint32_t job = warp; job < 2 * A.ranks; job += warps)
-	{
-		const uint32_t r = job >> 1;
-		if (r == run)
-			continue;
-		const uint32_t n = A.counts[r * A.lists + list];
-		const uint32_t* a = A.keys + (size_t)r * A.rankStride + A.offsets[r * A.lists + list];
-		const uint32_t key = (job & 1) ? lastKey : firstKey;
-		const uint32_t pos = r < run ? warpBound<true>(a, n, key) : warpBound<false>(a, n, key);
-		if (lane == 0)
-			((job & 1) ? sHi : sLo)[r] = pos;
-	}
-}
-// kStage = false (2-3 ranks): the brackets are searched in global memory — with one or two other runs the windows stay in
-// L1 and that measured faster than staging them (N=2: 0.07 vs 0.09 ms); kStage = true (>= 4 ranks) stages as described.
-template<bool kStage>
-__global__ void __launch_bounds__(kMergeThreads) kMergeSlice(const __grid_constant__ MergeArgs A)
-{
-	__shared__ uint32_t sLo[32], sHi[32], sOff[33];
-	__shared__ uint32_t sWin[kStage ? kMergeWindow : 1];
-	const uint32_t list = blockIdx.z, run = blockIdx.y;
-	const uint32_t lo = A.bounds[(list * A.ranks + run) * 2 + 0], hi = A.bounds[(list * A.ranks + run) * 2 + 1];
-	const uint32_t sliceStart = A.sliceInfo[list * 2 + 0];
-	const uint32_t* myKeys = A.keys + (size_t)run * A.rankStride + A.offsets[run * A.lists + list];
-	const uint32_t* myPays = A.payloads + (size_t)run * A.rankStride + A.offsets[run * A.lists + list];
-	const uint32_t outBase = A.outOffsets[list];
-	for (uint32_t i0 = lo + blockIdx.x * kMergeChunk; i0 < hi; i0 += gridDim.x * kMergeChunk)
-	{
-		const uint32_t i1 = min(i0 + kMergeChunk, hi);
-		__syncthreads(); // the previous chunk's readers are done with the shared arrays
-		if (threadIdx.x < A.ranks)
-			sLo[threadIdx.x] = sHi[threadIdx.x] = 0; // (the own run keeps an empty window)
-		__syncthreads();
-		bracketChunk(A, list, run, myKeys[i0], myKeys[i1 - 1], sLo, sHi);
-		__syncthreads();
-		if (threadIdx.x == 0)
-		{
-			uint32_t running = 0;
-			for (uint32_t r = 0; r < A.ranks; r++)
-			{
-				sOff[r] = running;
-				running += sHi[r] - sLo[r];
-			}
-			sOff[A.ranks] = running;
-		}
-		__syncthreads();
-		const bool staged = kStage && sOff[A.ranks] <= kMergeWindow; // block-uniform
-		if (staged)
-		{
-			for (uint32_t r = 0; r < A.ranks; r++)
-			{
-				const uint32_t* a = A.keys + (size_t)r * A.rankStride + A.offsets[r * A.lists + list] + sLo[r];
-				const uint32_t w = sHi[r] - sLo[r];
-				for (uint32_t j = threadIdx.x; j < w; j += kMergeThreads)
-					sWin[sOff[r] + j] = a[j];
-			}
-			__syncthreads();
-		}
-		for (uint32_t i = i0 + threadIdx.x; i < i1; i += kMergeThreads)
-		{
-			const uint32_t key = myKeys[i];
-			uint32_t pos = i;
-			for (uint32_t r = 0; r < A.ranks; r++)
-			{
-				if (r == run)
-					continue;
-				if (staged)
-				{
-					const uint32_t w = sHi[r] - sLo[r];
-					pos += sLo[r] + (r < run ? boundIn<true>(sWin + sOff[r], 0, w, key) : boundIn<false>(sWin + sOff[r], 0, w, key));
-				}
-				else
-				{
-					const uint32_t* a = A.keys + (size_t)r * A.rankStride + A.offsets[r * A.lists + list];
-					pos += r < run ? boundIn<true>(a, sLo[r], sHi[r], key) : boundIn<false>(a, sLo[r], sHi[r], key);
-				}
-			}
-			const uint32_t o = outBase + (pos - sliceStart);
-			A.outKeys[o] = key;
-			A.outPayloads[o] = myPays[i];
-			A.outRanks[o] = (uint8_t)run;
-		}
-	}
-}
-
-uint32_t launchMerge(cudaStream_t stream, const MergeArgs& A, uint32_t maxRunLength)
-{
-	if (A.lists == 0 || A.ranks == 0)
-		return 0;
-	kMergeBounds<<<A.lists, 32 * A.ranks, 0, stream>>>(A);
-	const uint32_t blocks = std::max(1u, std::min((maxRunLength / A.ranks + kMergeChunk - 1u) / kMergeChunk + 1u, 148u * 8u / std::max(1u, A.ranks)));
-	if (A.ranks <= 3)
-		kMergeSlice<false><<<dim3(blocks, A.ranks, A.lists), kMergeThreads, 0, stream>>>(A);
-	else
-		kMergeSlice<true><<<dim3(blocks, A.ranks, A.lists), kMergeThreads, 0, stream>>>(A);
-	return 2;
-}
-
-
 // ---- pairwise merge tree -------------------------------------------------------------------------------------------------
-// kMergeSlice ranks every element in every other run: ranks - 1 searches per element, which at 8 ranks costs more than the
-// sort that produced the runs. The tree merges the runs of a list two by two with merge-path partitioning instead:
-// ceil(log2 ranks) passes, each reading and writing every element of my slice once (9 bytes in, 9 out), whatever the rank
-// count. Level 1 reads the sub-ranges [lo, hi) of the received runs (the rank is implicit), the later levels read the
-// previous level from a scratch buffer; the groups of a list stay back to back in run order at every level, so the two
-// inputs of a merge are adjacent and its output covers exactly their union — one region per list, the same in the two
-// scratch buffers and in the final output. Ties go to the lower group (lower ranks hold lower global entity indices).
-constexpr uint32_t kTreeThreads = 256, kTreeItems = 8, kTreeTile = kTreeThreads * kTreeItems, kTreeMaxJobs = 1024;
+// The runs of a list are merged two by two with merge-path partitioning: ceil(log2 ranks) passes, each reading and writing
+// every element of my slice once (9 bytes in, 9 out), whatever the rank count. (Ranking every element in every other run
+// instead takes ranks - 1 searches per element, which at 8 ranks costs more than the sort that produced the runs.) Level 1
+// reads the sub-ranges [lo, hi) of the received runs (the rank is implicit), the later levels read the previous level from
+// a scratch buffer; the groups of a list stay back to back in run order at every level, so the two inputs of a merge are
+// adjacent and its output covers exactly their union — one region per list, the same in the two scratch buffers and in the
+// final output. Ties go to the lower group (lower ranks hold lower global entity indices).
+constexpr uint32_t kTreeThreads = 256, kTreeItems = 8, kTreeTile = kTreeThreads * kTreeItems;
+// one job per (list, pair of runs) at level 1: every list the layout allows at the largest rank count
+constexpr uint32_t kTreeMaxJobs = kMaxViews * kMaxPools * 16;
+static_assert(kTreeMaxJobs >= kMaxViews * kMaxPools * ((kMaxRanks + 1) / 2), "the job table must hold every list at kMaxRanks ranks");
 // shared arrays skip one word in 33: a thread's outputs are kTreeItems apart from its neighbour's, which would put
 // every fourth lane into the same bank
 constexpr uint32_t kTreePadded = kTreeTile + kTreeTile / 32, kTreeBlocksPerSM = 4;
@@ -675,7 +553,7 @@ __global__ void kMergePlan(const uint32_t* __restrict__ gathered, uint32_t block
 		uint32_t e = sError;
 		if (running > outCapacity)
 		{
-			// nothing may be written: drop every run (kMergeBounds / kMergeSlice then see empty lists)
+			// nothing may be written: drop every run (kMergeBounds and the tree then see empty lists)
 			e |= 4u;
 			for (uint32_t i = 0; i < ranks * lists; i++)
 				counts[i] = 0;
@@ -689,22 +567,6 @@ __global__ void kMergePlan(const uint32_t* __restrict__ gathered, uint32_t block
 
 using namespace gsp;
 
-extern "C" int gsp_merge_gathered(void* cudaStream, uint32_t ranks, uint32_t myRank, uint32_t lists, uint32_t rankStride,
-	const uint32_t* dKeys, const uint32_t* dPayloads, const uint32_t* dOffsets, const uint32_t* dCounts, uint32_t maxRunLength,
-	uint32_t* dBounds, uint32_t* dSliceInfo, uint32_t* dOutKeys, uint32_t* dOutPayloads, uint8_t* dOutRanks,
-	const uint32_t* dOutOffsets)
-{
-	if (ranks == 0 || ranks > 32 || myRank >= ranks || !dKeys || !dPayloads || !dOffsets || !dCounts || !dBounds ||
-		!dSliceInfo || !dOutKeys || !dOutPayloads || !dOutRanks || !dOutOffsets)
-		return GSP_ERR_INVALID;
-	MergeArgs A;
-	A.keys = dKeys; A.payloads = dPayloads; A.offsets = dOffsets; A.counts = dCounts; A.bounds = dBounds;
-	A.sliceInfo = dSliceInfo; A.outKeys = dOutKeys; A.outPayloads = dOutPayloads; A.outRanks = dOutRanks;
-	A.outOffsets = dOutOffsets; A.rankStride = rankStride; A.ranks = ranks; A.lists = lists; A.myRank = myRank; A.preSplit = 0;
-	launchMerge((cudaStream_t)cudaStream, A, maxRunLength);
-	return cudaGetLastError() == cudaSuccess ? GSP_OK : GSP_ERR_CUDA;
-}
-
 extern "C" uint32_t gsp_exchange_block_words(uint32_t capacityElems)
 {
 	return kExHeaderWords + 2u * capacityElems;
@@ -717,7 +579,8 @@ extern "C" uint32_t gsp_merge_plan_words(uint32_t ranks, uint32_t lists)
 
 namespace gsp
 {
-// plan + bounds + merge of `ranks` packed blocks (block r at r * (kExHeaderWords + 2 * capacityElems) words)
+// plan + bounds + merge of `ranks` packed blocks (block r at r * (kExHeaderWords + 2 * capacityElems) words).
+// Preconditions: lists * ceil(ranks / 2) <= kTreeMaxJobs, exchangeBlocksIndexable(capacityElems, ranks).
 uint32_t launchMergePacked(cudaStream_t stream, uint32_t ranks, uint32_t myRank, uint32_t lists, uint32_t capacityElems,
 	const uint32_t* dGathered, uint32_t* dPlan, uint32_t* dSliceInfo, uint32_t* dOutKeys, uint32_t* dOutPays, uint8_t* dOutRanks,
 	uint32_t outCapacity, bool preSplit, uint32_t* dTreeScratch, uint32_t smCount)
@@ -730,15 +593,11 @@ uint32_t launchMergePacked(cudaStream_t stream, uint32_t ranks, uint32_t myRank,
 	A.outOffsets = dPlan + 2 * ranks * lists; A.bounds = dPlan + 2 * ranks * lists + lists;
 	A.sliceInfo = dSliceInfo; A.outKeys = dOutKeys; A.outPayloads = dOutPays; A.outRanks = dOutRanks;
 	A.rankStride = blockWords; A.ranks = ranks; A.lists = lists; A.myRank = myRank; A.preSplit = preSplit ? 1u : 0u;
-	if (dTreeScratch && lists * ((ranks + 1) / 2) <= kTreeMaxJobs && (uint64_t)blockWords * ranks < 0xFFFFFFFFull)
-		return 1 + launchMergeTree(stream, A, outCapacity, dTreeScratch, smCount);
-	// (pre-split runs are merged whole: size the grid for a full block per run)
-	return 1 + launchMerge(stream, A, preSplit ? (uint32_t)std::min<uint64_t>((uint64_t)capacityElems * ranks, 0xFFFFFFFFull) : capacityElems);
+	return 1 + launchMergeTree(stream, A, outCapacity, dTreeScratch, smCount);
 }
 
 // ---- all-to-all protocol: common splitters from samples, one sub-block per destination --------------------------------------
 constexpr uint32_t kSamples = 64, kSampleWords = kSamples + 1; // (exchange.cu: kExSamples)
-constexpr uint32_t kPackMaxRanks = 32;
 
 // samples[list][k] = key at position (2k + 1) * count / (2 * kSamples) of my sorted run, samples[list][kSamples] = count
 __global__ void kSampleRuns(const SegmentDev* __restrict__ segments, const uint32_t* __restrict__ counters,
@@ -781,7 +640,7 @@ __global__ void __launch_bounds__(1024) kSplitRuns(const __grid_constant__ Split
 		bounds[0] = 0; bounds[A.ranks] = myCount;
 	}
 	// every rank's samples of this list into shared memory (the value search below probes them ~200 times per lane)
-	__shared__ uint32_t sSamples[kPackMaxRanks][kSampleWords];
+	__shared__ uint32_t sSamples[kMaxRanks][kSampleWords];
 	for (uint32_t i = threadIdx.x; i < A.ranks * kSampleWords; i += blockDim.x)
 		sSamples[i / kSampleWords][i % kSampleWords] = A.gathered[((size_t)(i / kSampleWords) * A.lists + l) * kSampleWords + i % kSampleWords];
 	__syncthreads();
@@ -822,7 +681,7 @@ __global__ void __launch_bounds__(1024) kSplitRuns(const __grid_constant__ Split
 		if (w >= target) hi = mid; else lo = mid + 1;
 	}
 	const uint32_t splitter = totalWeight ? lo : 0xFFFFFFFFu;
-	const uint32_t pos = warpBound<false>(A.keys + sg.offset, myCount, splitter); // keys equal to a splitter start the next range
+	const uint32_t pos = warpBound(A.keys + sg.offset, myCount, splitter); // keys equal to a splitter start the next range
 	if (lane == 0)
 	{
 		A.splitters[l * (A.ranks - 1) + (j - 1)] = splitter;
@@ -842,8 +701,8 @@ struct PackArgs
 };
 __global__ void __launch_bounds__(256) kPackByDestination(const __grid_constant__ PackArgs A)
 {
-	__shared__ uint32_t sBound[kPackMaxRanks + 1];
-	__shared__ uint32_t sTotal[kPackMaxRanks], sBefore[kPackMaxRanks]; // per destination: all lists / the lists before this one
+	__shared__ uint32_t sBound[kMaxRanks + 1];
+	__shared__ uint32_t sTotal[kMaxRanks], sBefore[kMaxRanks]; // per destination: all lists / the lists before this one
 	const size_t blockWords = kExHeaderWords + 2ull * A.capacity;
 	if (threadIdx.x < A.ranks)
 	{
@@ -945,18 +804,6 @@ uint32_t launchSliceStarts(cudaStream_t stream, uint32_t ranks, uint32_t lists, 
 }
 } // namespace gsp
 
-extern "C" int gsp_merge_gathered_packed(void* cudaStream, uint32_t ranks, uint32_t myRank, uint32_t lists, uint32_t capacityElems,
-	const uint32_t* dGathered, uint32_t* dPlan, uint32_t* dSliceInfo, uint32_t* dOutKeys, uint32_t* dOutPayloads,
-	uint8_t* dOutRanks, uint32_t outCapacity)
-{
-	if (ranks == 0 || ranks > 32 || myRank >= ranks || lists == 0 || lists > kExMaxLists || !dGathered || !dPlan || !dSliceInfo ||
-		!dOutKeys || !dOutPayloads || !dOutRanks)
-		return GSP_ERR_INVALID;
-	gsp::launchMergePacked((cudaStream_t)cudaStream, ranks, myRank, lists, capacityElems, dGathered, dPlan, dSliceInfo, dOutKeys,
-		dOutPayloads, dOutRanks, outCapacity, false, nullptr, 0);
-	return cudaGetLastError() == cudaSuccess ? GSP_OK : GSP_ERR_CUDA;
-}
-
 extern "C" uint64_t gsp_merge_tree_scratch_words(uint32_t outCapacity)
 {
 	return gsp::mergeTreeScratchWords(outCapacity);
@@ -966,8 +813,9 @@ extern "C" int gsp_merge_gathered_packed_tree(void* cudaStream, uint32_t ranks, 
 	const uint32_t* dGathered, uint32_t* dPlan, uint32_t* dSliceInfo, uint32_t* dOutKeys, uint32_t* dOutPayloads,
 	uint8_t* dOutRanks, uint32_t outCapacity, uint32_t* dScratch)
 {
-	if (ranks == 0 || ranks > 32 || myRank >= ranks || lists == 0 || lists > kExMaxLists || !dGathered || !dPlan || !dSliceInfo ||
-		!dOutKeys || !dOutPayloads || !dOutRanks || !dScratch || lists * ((ranks + 1) / 2) > 1024u)
+	if (ranks == 0 || ranks > kMaxRanks || myRank >= ranks || lists == 0 || lists > kExMaxLists || !dGathered || !dPlan ||
+		!dSliceInfo || !dOutKeys || !dOutPayloads || !dOutRanks || !dScratch || lists * ((ranks + 1) / 2) > gsp::kTreeMaxJobs ||
+		!exchangeBlocksIndexable(capacityElems, ranks))
 		return GSP_ERR_INVALID;
 	int device = 0, sms = 148;
 	cudaGetDevice(&device);

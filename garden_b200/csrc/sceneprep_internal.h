@@ -249,6 +249,13 @@ constexpr uint32_t kSortTile = kSortItems * kSortThreads;
 // ---- packed exchange block of the multi-GPU path (merge.cu) ----
 constexpr uint32_t kExHeaderWords = 256, kExHeaderFixed = 8, kExMaxLists = kExHeaderWords - kExHeaderFixed;
 constexpr uint32_t kExMagic = 0x47535031u; // "GSP1"
+constexpr uint32_t kMaxRanks = 32;          // GPUs of one communicator (gsp_comm_init)
+// The merge tree (merge.cu) indexes the received blocks with 32-bit element indices: the `ranks` blocks of
+// kExHeaderWords + 2 * capacityElems words each must stay below 2^32 words together.
+inline bool exchangeBlocksIndexable(uint32_t capacityElems, uint32_t ranks)
+{
+	return ((uint64_t)kExHeaderWords + 2ull * capacityElems) * ranks < (1ull << 32);
+}
 
 // ---- kernel launchers (each returns the number of kernels it launched, or throws nothing; errors via cudaGetLastError) ----
 uint32_t launchStageTransforms(Context& c, const void* dAos, uint32_t stride, uint32_t first, uint32_t count, bool full,

@@ -13,8 +13,6 @@
 // earlier pass or frame simply reads as "not published yet".
 #include "sceneprep_internal.h"
 #include <algorithm>
-#include <cstdlib>
-#include <cstring>
 
 namespace gsp
 {
@@ -94,7 +92,6 @@ __device__ __forceinline__ uint32_t ballotPeers(uint32_t peers, uint32_t digit, 
 constexpr uint32_t kSortBlocksPerSM = GSP_SORT_BLOCKS_PER_SM; // resident blocks the pass is sized for
 constexpr uint32_t kLookbackBatch = 4; // predecessor tiles inspected per step (independent loads in flight; 16 measured slower, 8 / 4 / 2 within 2 %)
 
-template<bool kUseMatch>
 __global__ void __launch_bounds__(kSortThreads, kSortBlocksPerSM) kSortPass(const __grid_constant__ SortArgs A, uint32_t pass, uint32_t epoch,
 	const uint32_t* __restrict__ keysIn, const uint32_t* __restrict__ payIn,
 	uint32_t* __restrict__ keysOut, uint32_t* __restrict__ payOut)
@@ -176,14 +173,9 @@ __global__ void __launch_bounds__(kSortThreads, kSortBlocksPerSM) kSortPass(cons
 		{
 			const uint32_t dg = (key[i] >> shift) & (kRadix - 1);
 			uint32_t peers = 0xffffffffu;
-			if (kUseMatch)
-				peers = __match_any_sync(0xffffffffu, dg);
-			else
-			{
-				#pragma unroll
-				for (uint32_t b = 0; b < kRadixBits; b++)
-					peers = ballotPeers(peers, dg, 1u << b);
-			}
+			#pragma unroll
+			for (uint32_t b = 0; b < kRadixBits; b++)
+				peers = ballotPeers(peers, dg, 1u << b);
 			peerMask[i] = peers;
 		}
 		#pragma unroll
@@ -305,10 +297,7 @@ uint32_t launchSort(Context& c, cudaEvent_t afterHistogram)
 	{
 		const uint32_t in = pass & 1, out = in ^ 1;
 		if (++c.sortEpoch == 0) ++c.sortEpoch; // 0 is what freshly allocated (zeroed) status memory holds
-		// the lanes holding the same digit: eight ballots (default) or one match.any (GSP_SORT_MATCH=1, for A/B measurements)
-		static const bool useMatch = []{ const char* e = getenv("GSP_SORT_MATCH"); return e && !strcmp(e, "1"); }();
-		if (useMatch) kSortPass<true><<<passGrid, kSortThreads, 0, c.stream>>>(A, pass, c.sortEpoch, c.keys[in], c.payloads[in], c.keys[out], c.payloads[out]);
-		else kSortPass<false><<<passGrid, kSortThreads, 0, c.stream>>>(A, pass, c.sortEpoch, c.keys[in], c.payloads[in], c.keys[out], c.payloads[out]);
+		kSortPass<<<passGrid, kSortThreads, 0, c.stream>>>(A, pass, c.sortEpoch, c.keys[in], c.payloads[in], c.keys[out], c.payloads[out]);
 		launches++;
 	}
 	return launches; // 4 passes: sorted data ends in buffer 0

@@ -6,8 +6,7 @@ ties broken by global entity order (ranks hold contiguous ranges in rank order, 
 
 The exchange itself lives in libgarden_sceneprep.so (csrc/exchange.cu, csrc/merge.cu: NCCL loaded by the library, no host
 synchronisation, key-range all-to-all + merge-path tree) — `PipelinedRunMerger` below only carries the NCCL unique id over
-torch.distributed and forwards to gsp_exchange_*. `RunMerger` is round 1's host-synchronous path (lengths to the host, two
-all-gathers through torch.distributed, gsp_merge_gathered), kept for tools/dist_parity.py's cross-check.
+torch.distributed and forwards to gsp_exchange_*.
 
 `plan_gather`, `pack_block`, `plan_from_blocks`, `sample_run`, `common_splitters`, `split_bounds` and `merge_reference` are
 pure numpy statements of what the device kernels compute (layouts, splitters, expected merges); the CPU tests check them,
@@ -208,83 +207,6 @@ def exchange_counts(counts: np.ndarray, group=None) -> np.ndarray:
     out = torch.empty(world * mine.numel(), dtype=torch.int64, device=device)
     dist.all_gather_into_tensor(out, mine, group=group)
     return out.cpu().numpy().reshape(world, mine.numel())
-
-
-class RunMerger:
-    """Gather + merge of one ScenePrep's sorted runs across the ranks of the default process group (NCCL)."""
-
-    launches_per_frame = 2  # kMergeBounds + kMergeSlice
-
-    def __init__(self, sp):
-        import torch
-        import torch.distributed as dist
-        self.torch, self.dist = torch, dist
-        self.sp = sp
-        self.rank, self.world = dist.get_rank(), dist.get_world_size()
-        self.dev = torch.device("cuda", torch.cuda.current_device())
-        self.send_keys = self.send_pays = None
-        self.gk = self.gp = None
-        self.out_keys = self.out_pays = self.out_ranks = None
-        self.bounds = self.slice_info = None
-        self.last = None
-
-    def _ensure(self, name: str, n: int, dtype):
-        t = getattr(self, name)
-        if t is None or t.numel() < n:
-            t = self.torch.empty(max(int(n * 1.25), 16), dtype=dtype, device=self.dev)
-            setattr(self, name, t)
-        return t
-
-    def gather_and_merge(self):
-        """Must be called after sp.run_async(); leaves this rank's merged slices on the device.
-        Returns dict(counts, totals, slice_info (device tensor [lists, 2]))."""
-        torch, dist, sp = self.torch, self.dist, self.sp
-        sp.sync()  # list lengths are needed on the host to size the exchange
-        counts = sp.list_counts().astype(np.int64)
-        lists = counts.size
-        all_counts = exchange_counts(counts)
-        offsets, stride, out_offsets, totals = plan_gather(all_counts)
-        send_k = self._ensure("send_keys", stride, torch.int32)
-        send_p = self._ensure("send_pays", stride, torch.int32)
-        sp.export_runs(send_k.data_ptr(), send_p.data_ptr(), stride)
-        # the export runs on the context's stream, the all-gathers below on torch's current stream: this (already
-        # host-synchronous) path simply waits for the export, whatever stream the context was given
-        sp.sync()
-        gk = self._ensure("gk", stride * self.world, torch.int32)
-        gp = self._ensure("gp", stride * self.world, torch.int32)
-        dist.all_gather_into_tensor(gk[: stride * self.world], send_k[:stride])
-        dist.all_gather_into_tensor(gp[: stride * self.world], send_p[:stride])
-        total = int(totals.sum())
-        out_k = self._ensure("out_keys", total, torch.int32)
-        out_p = self._ensure("out_pays", total, torch.int32)
-        out_r = self._ensure("out_ranks", total, torch.uint8)
-        bounds = self._ensure("bounds", lists * self.world * 2, torch.int32)
-        sinfo = self._ensure("slice_info", lists * 2, torch.int32)
-        meta = torch.as_tensor(np.concatenate([offsets.reshape(-1), all_counts.astype(np.uint32).reshape(-1),
-                                               out_offsets]).astype(np.int64), device=self.dev).to(torch.int32)
-        n_rl = self.world * lists
-        d_off, d_cnt, d_out_off = meta[:n_rl], meta[n_rl:2 * n_rl], meta[2 * n_rl:]
-        stream = torch.cuda.current_stream().cuda_stream
-        rc = sp.lib.gsp_merge_gathered(stream, self.world, self.rank, lists, stride, gk.data_ptr(), gp.data_ptr(),
-                                       d_off.data_ptr(), d_cnt.data_ptr(), int(all_counts.max()), bounds.data_ptr(),
-                                       sinfo.data_ptr(), out_k.data_ptr(), out_p.data_ptr(), out_r.data_ptr(),
-                                       d_out_off.data_ptr())
-        if rc != 0:
-            raise RuntimeError(f"gsp_merge_gathered failed with {rc}")
-        self.last = {"counts": all_counts, "totals": totals, "out_offsets": out_offsets, "slice_info": sinfo[: lists * 2],
-                     "meta": meta, "bytes_gathered": int(stride * self.world * 8)}
-        return self.last
-
-    def slices_to_host(self):
-        """Downloads this rank's merged slices: list of (start, keys, payloads, ranks) per list (for tests)."""
-        info = self.last["slice_info"].cpu().numpy().astype(np.uint32).reshape(-1, 2)
-        out = []
-        for l, (start, length) in enumerate(info):
-            o = int(self.last["out_offsets"][l])
-            sl = slice(o, o + int(length))
-            out.append((int(start), self.out_keys[sl].cpu().numpy().view(np.uint32),
-                        self.out_pays[sl].cpu().numpy().view(np.uint32), self.out_ranks[sl].cpu().numpy()))
-        return out
 
 
 class PipelinedRunMerger:

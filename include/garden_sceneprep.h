@@ -162,36 +162,29 @@ int gsp_get_sorted_run_device(gsp_context* ctx, uint32_t view, int listKind, uin
 uint32_t gsp_list_count(const gsp_context* ctx);
 /* Length of every list of the last completed frame (`capacity` >= gsp_list_count entries). */
 int gsp_get_list_counts(gsp_context* ctx, uint32_t* counts, uint32_t capacity);
-/* Packs the sorted (key, payload) runs of all lists back to back into caller-provided DEVICE buffers (the send buffers of
- * the NCCL all-gather). Enqueued on the context's stream. */
+/* Packs the sorted (key, payload) runs of all lists back to back into caller-provided DEVICE buffers (list l follows list
+ * l - 1, lengths as gsp_get_list_counts). Enqueued on the context's stream. */
 int gsp_export_runs(gsp_context* ctx, uint32_t* dKeys, uint32_t* dPayloads, uint32_t capacity);
-/* K-way merge after the all-gather: this rank merges ITS key range of every list out of the `ranks` gathered runs
- * (splitters = quantiles of rank 0's run, identical on every rank). All pointers are device pointers.
- *   dKeys/dPayloads: gathered buffers, rank r's block at r * rankStride; dOffsets/dCounts: [ranks][lists];
- *   dBounds: [lists][ranks][2] scratch; dSliceInfo: [lists][2] out = (global position of my slice, slice length);
- *   dOutKeys/dOutPayloads/dOutRanks: my slices, list l at dOutOffsets[l]. Ties resolve to (rank, payload) order. */
-int gsp_merge_gathered(void* cudaStream, uint32_t ranks, uint32_t myRank, uint32_t lists, uint32_t rankStride,
-	const uint32_t* dKeys, const uint32_t* dPayloads, const uint32_t* dOffsets, const uint32_t* dCounts, uint32_t maxRunLength,
-	uint32_t* dBounds, uint32_t* dSliceInfo, uint32_t* dOutKeys, uint32_t* dOutPayloads, uint8_t* dOutRanks,
-	const uint32_t* dOutOffsets);
-
-/* Host-synchronisation-free variant of the same exchange. A frame only has to be ENQUEUED (gsp_run_async): list lengths are
- * read on the device. Every rank fills one fixed-capacity block
+/* The multi-GPU exchange step without host synchronisation. A frame only has to be ENQUEUED (gsp_run_async): list lengths
+ * are read on the device. Every rank fills one fixed-capacity block
  *   [0, 256) header { magic, lists, total, capacity, overflow, 0, 0, 0, count[lists] } | keys[capacity] | payloads[capacity]
- * (gsp_exchange_block_words(capacity) 32-bit words), ONE all-gather of equal blocks moves everything, and the merge plans
- * itself from the gathered headers. dPlan = gsp_merge_plan_words(ranks, lists) words of device scratch; its last 8 words
- * are flags the caller reads back whenever convenient: { error bits (1 a block overflowed its capacity, 2 bad header,
- * 4 merged lists exceed outCapacity), merged total, largest per-rank total, 0... }. With a non-zero error word nothing was
- * merged: grow the capacity to hold flags[2] (or outCapacity to hold flags[1]) and repeat the frame. */
+ * (gsp_exchange_block_words(capacity) 32-bit words) with gsp_export_runs_packed, and ONE all-gather of equal blocks moves
+ * everything. */
 uint32_t gsp_exchange_block_words(uint32_t capacityElems);
 uint32_t gsp_merge_plan_words(uint32_t ranks, uint32_t lists);
 int gsp_export_runs_packed(gsp_context* ctx, uint32_t* dBlock, uint32_t capacityElems);
-int gsp_merge_gathered_packed(void* cudaStream, uint32_t ranks, uint32_t myRank, uint32_t lists, uint32_t capacityElems,
-	const uint32_t* dGathered, uint32_t* dPlan, uint32_t* dSliceInfo, uint32_t* dOutKeys, uint32_t* dOutPayloads,
-	uint8_t* dOutRanks, uint32_t outCapacity);
-/* The same merge as a pairwise merge-path tree (ceil(log2 ranks) passes over my slice instead of ranks - 1 searches per
- * element; what gsp_exchange_async uses). dScratch = gsp_merge_tree_scratch_words(outCapacity) 32-bit words. Refused
- * (GSP_ERR_INVALID) when lists * ceil(ranks / 2) exceeds 1024. */
+/* K-way merge of the `ranks` gathered blocks (block r at r * gsp_exchange_block_words(capacityElems) words): this rank merges
+ * ITS key range of every list (splitters = quantiles of the longest run, identical on every rank) with a pairwise
+ * merge-path tree, ceil(log2 ranks) passes over its slice; what gsp_exchange_async uses. The merge plans itself from the
+ * gathered headers. All pointers are device pointers. dPlan = gsp_merge_plan_words(ranks, lists) words of device scratch;
+ * its last 8 words are flags the caller reads back whenever convenient: { error bits (1 a block overflowed its capacity,
+ * 2 bad header, 4 merged lists exceed outCapacity), merged total, largest per-rank total, 0... }. With a non-zero error
+ * word nothing was merged: grow the capacity to hold flags[2] (or outCapacity to hold flags[1]) and repeat the frame.
+ * dSliceInfo: [lists][2] out = (global position of my slice, slice length); dOutKeys/dOutPayloads/dOutRanks: my slices,
+ * list l at the merged list's offset (plan words [2 * ranks * lists, + lists)). Ties resolve to (rank, payload) order.
+ * dScratch = gsp_merge_tree_scratch_words(outCapacity) 32-bit words. Refused (GSP_ERR_INVALID) when ranks exceeds 32,
+ * lists exceeds 248, lists * ceil(ranks / 2) exceeds 2048 (every layout of up to 128 lists at 32 ranks fits), or the
+ * gathered blocks reach 2^32 words: (256 + 2 * capacityElems) * ranks >= 2^32. */
 uint64_t gsp_merge_tree_scratch_words(uint32_t outCapacity);
 int gsp_merge_gathered_packed_tree(void* cudaStream, uint32_t ranks, uint32_t myRank, uint32_t lists, uint32_t capacityElems,
 	const uint32_t* dGathered, uint32_t* dPlan, uint32_t* dSliceInfo, uint32_t* dOutKeys, uint32_t* dOutPayloads,
@@ -209,7 +202,7 @@ int gsp_merge_gathered_packed_tree(void* cudaStream, uint32_t ranks, uint32_t my
  * GSP_EXCHANGE=allgather|alltoall selects the protocol (default alltoall: runs are cut by common, sample-based splitters
  * before they travel, every rank receives only the key range it merges: two collectives per frame — a small all-gather of
  * samples and grouped send/recv of the sub-blocks, whose headers also carry where each slice starts; falls back to allgather
- * beyond 124 lists). GSP_MERGE=slice selects gsp_merge_gathered's rank-in-every-run merge instead of the merge-path tree. */
+ * beyond 124 lists). Both protocols merge with gsp_merge_gathered_packed_tree's merge-path tree. */
 #define GSP_COMM_ID_BYTES 128
 int gsp_comm_unique_id(uint8_t id[GSP_COMM_ID_BYTES]);
 int gsp_comm_init(gsp_context* ctx, const uint8_t id[GSP_COMM_ID_BYTES], uint32_t ranks, uint32_t rank);

@@ -31,78 +31,6 @@ def _runs_to_host(sp, torch):
     return counts, k[:total].cpu().numpy().view(np.uint32), p[:total].cpu().numpy().view(np.uint32)
 
 
-@pytest.mark.parametrize("ranks", [2, 3])
-def test_emulated_ranks_merge_equals_single_sort(sceneprep_lib, ranks):
-    import torch
-    from garden_b200.binding import ScenePrep
-    chains, depth = 3000, 4
-    n = chains * (depth + 1)
-    box = (-150, -10, -150, 150, 10, 150)
-    whole = scenes.make_scene(n, depth, 5, box)
-    whole.camera_pos = np.array([2.0, 1.0, -3.0], np.float32)
-    views, _ = V.camera_and_cascades(0.3, -0.1, 1.2, 16 / 9, 0.01, 100.0, (0.05, 0.1, 0.25, 1.0))
-    sp = ScenePrep(0)
-    _prepare(sp, whole, views)
-    full_counts, full_k, full_p = _runs_to_host(sp, torch)
-    lists = full_counts.size
-
-    # shards: contiguous entity ranges cut at chain boundaries
-    per = (chains // ranks) * (depth + 1)
-    starts = [r * per for r in range(ranks)] + [n]
-    shard_runs = []
-    for r in range(ranks):
-        a, b = starts[r], starts[r + 1]
-        sc = scenes.SceneDesc(whole.position[a:b], whole.rotation[a:b], whole.scale[a:b],
-                              np.where(whole.parent[a:b] >= 0, whole.parent[a:b] - a, -1).astype(np.int32), whole.tflags[a:b],
-                              [scenes.PoolDesc(whole.pools[0].render_type, np.arange(b - a, dtype=np.uint32), whole.pools[0].aabb[a:b])],
-                              None, whole.camera_pos)
-        _prepare(sp, sc, views)
-        shard_runs.append(_runs_to_host(sp, torch))
-
-    all_counts = np.stack([c for c, _, _ in shard_runs])
-    assert np.array_equal(all_counts.sum(axis=0), full_counts)
-    offsets, stride, out_offsets, totals = plan_gather(all_counts)
-    gk = torch.zeros(stride * ranks, dtype=torch.int32, device="cuda")
-    gp = torch.zeros(stride * ranks, dtype=torch.int32, device="cuda")
-    for r, (c, k, p) in enumerate(shard_runs):
-        gk[r * stride: r * stride + k.size] = torch.from_numpy(k.view(np.int32)).cuda()
-        gp[r * stride: r * stride + p.size] = torch.from_numpy(p.view(np.int32)).cuda()
-    meta = torch.from_numpy(np.concatenate([offsets.reshape(-1), all_counts.astype(np.uint32).reshape(-1), out_offsets]).astype(np.int32)).cuda()
-    nrl = ranks * lists
-    total = int(totals.sum())
-    merged_k = np.zeros(total, np.uint32); merged_p = np.zeros(total, np.uint32); merged_r = np.zeros(total, np.uint8)
-    covered = np.zeros(total, bool)
-    for me in range(ranks):
-        out_k = torch.zeros(total, dtype=torch.int32, device="cuda"); out_p = torch.zeros_like(out_k)
-        out_r = torch.zeros(total, dtype=torch.uint8, device="cuda")
-        bounds = torch.zeros(lists * ranks * 2, dtype=torch.int32, device="cuda")
-        sinfo = torch.zeros(lists * 2, dtype=torch.int32, device="cuda")
-        rc = sp.lib.gsp_merge_gathered(0, ranks, me, lists, stride, gk.data_ptr(), gp.data_ptr(), meta[:nrl].data_ptr(),
-                                       meta[nrl:2 * nrl].data_ptr(), int(all_counts.max()), bounds.data_ptr(), sinfo.data_ptr(),
-                                       out_k.data_ptr(), out_p.data_ptr(), out_r.data_ptr(), meta[2 * nrl:].data_ptr())
-        assert rc == 0
-        torch.cuda.synchronize()
-        info = sinfo.cpu().numpy().reshape(lists, 2)
-        ok, op, orr = out_k.cpu().numpy().view(np.uint32), out_p.cpu().numpy().view(np.uint32), out_r.cpu().numpy()
-        for l in range(lists):
-            start, length = int(info[l, 0]), int(info[l, 1])
-            runs_k = [shard_runs[r][1][offsets[r, l]: offsets[r, l] + all_counts[r, l]] for r in range(ranks)]
-            runs_p = [shard_runs[r][2][offsets[r, l]: offsets[r, l] + all_counts[r, l]] for r in range(ranks)]
-            ek, ep, er, estart = merge_reference(runs_k, runs_p, my_rank=me)
-            assert (start, length) == (estart, ek.size), f"rank {me} list {l}: slice bounds"
-            o = int(out_offsets[l])
-            assert np.array_equal(ok[o:o + length], ek) and np.array_equal(op[o:o + length], ep) and np.array_equal(orr[o:o + length], er)
-            g = slice(o + start, o + start + length)
-            assert not covered[g].any()
-            covered[g] = True
-            merged_k[g], merged_p[g], merged_r[g] = ek, ep, er
-    assert covered.all()
-    # the merged order equals the single-GPU sort of the whole scene (payload = pool << 28 | slot, slot shifted by the shard start)
-    global_p = (merged_p & 0xF0000000) | ((merged_p & 0x0FFFFFFF) + np.array(starts, np.uint32)[merged_r])
-    assert np.array_equal(merged_k, full_k)
-    assert np.array_equal(global_p, full_p)
-
-
 def _shards(whole, ranks, chains, depth):
     n = whole.entity_count
     per = (chains // ranks) * (depth + 1)
@@ -117,9 +45,9 @@ def _shards(whole, ranks, chains, depth):
     return out, starts
 
 
-@pytest.mark.parametrize("ranks,tree", [(2, False), (4, False), (8, False), (1, True), (2, True), (3, True), (4, True), (5, True), (8, True)])
-def test_packed_exchange_emulated_ranks(sceneprep_lib, ranks, tree):
-    """The host-synchronisation-free exchange (gsp_export_runs_packed -> [all-gather] -> gsp_merge_gathered_packed):
+@pytest.mark.parametrize("ranks", [1, 2, 3, 4, 5, 6, 7, 8, 16])
+def test_packed_exchange_emulated_ranks(sceneprep_lib, ranks):
+    """The host-synchronisation-free exchange (gsp_export_runs_packed -> [all-gather] -> gsp_merge_gathered_packed_tree):
     blocks are exported right after gsp_run_async (no gsp_sync), laid out as the all-gather would, merged per rank, and
     checked against the numpy merge and against a single sort of the whole scene. Then the overflow protocol."""
     import torch
@@ -164,13 +92,10 @@ def test_packed_exchange_emulated_ranks(sceneprep_lib, ranks, tree):
         out_k = torch.zeros(total, dtype=torch.int32, device="cuda"); out_p = torch.zeros_like(out_k)
         out_r = torch.zeros(total, dtype=torch.uint8, device="cuda")
         sinfo = torch.zeros(lists * 2, dtype=torch.int32, device="cuda")
-        if tree:  # the pairwise merge-path tree gsp_exchange_async uses; scratch poisoned so stale reads would show
-            scratch = torch.full((int(lib.gsp_merge_tree_scratch_words(total)),), -1, dtype=torch.int32, device="cuda")
-            rc = lib.gsp_merge_gathered_packed_tree(0, ranks, me, lists, cap, gathered.data_ptr(), plan.data_ptr(), sinfo.data_ptr(),
-                                                    out_k.data_ptr(), out_p.data_ptr(), out_r.data_ptr(), total, scratch.data_ptr())
-        else:
-            rc = lib.gsp_merge_gathered_packed(0, ranks, me, lists, cap, gathered.data_ptr(), plan.data_ptr(), sinfo.data_ptr(),
-                                               out_k.data_ptr(), out_p.data_ptr(), out_r.data_ptr(), total)
+        # (scratch poisoned so stale reads would show)
+        scratch = torch.full((int(lib.gsp_merge_tree_scratch_words(total)),), -1, dtype=torch.int32, device="cuda")
+        rc = lib.gsp_merge_gathered_packed_tree(0, ranks, me, lists, cap, gathered.data_ptr(), plan.data_ptr(), sinfo.data_ptr(),
+                                                out_k.data_ptr(), out_p.data_ptr(), out_r.data_ptr(), total, scratch.data_ptr())
         assert rc == 0
         torch.cuda.synchronize()
         pl = plan.cpu().numpy().view(np.uint32)
@@ -208,13 +133,9 @@ def test_packed_exchange_emulated_ranks(sceneprep_lib, ranks, tree):
     sentinel = torch.full((total,), 0x5a5a5a5a, dtype=torch.int32, device="cuda")
     out_p = sentinel.clone(); out_r = torch.zeros(total, dtype=torch.uint8, device="cuda")
     sinfo = torch.zeros(lists * 2, dtype=torch.int32, device="cuda")
-    if tree:
-        scratch = torch.zeros(int(lib.gsp_merge_tree_scratch_words(total)), dtype=torch.int32, device="cuda")
-        rc = lib.gsp_merge_gathered_packed_tree(0, ranks, 0, lists, small, g2.data_ptr(), plan.data_ptr(), sinfo.data_ptr(),
-                                                sentinel.data_ptr(), out_p.data_ptr(), out_r.data_ptr(), total, scratch.data_ptr())
-    else:
-        rc = lib.gsp_merge_gathered_packed(0, ranks, 0, lists, small, g2.data_ptr(), plan.data_ptr(), sinfo.data_ptr(),
-                                           sentinel.data_ptr(), out_p.data_ptr(), out_r.data_ptr(), total)
+    scratch = torch.zeros(int(lib.gsp_merge_tree_scratch_words(total)), dtype=torch.int32, device="cuda")
+    rc = lib.gsp_merge_gathered_packed_tree(0, ranks, 0, lists, small, g2.data_ptr(), plan.data_ptr(), sinfo.data_ptr(),
+                                            sentinel.data_ptr(), out_p.data_ptr(), out_r.data_ptr(), total, scratch.data_ptr())
     assert rc == 0
     sp.sync()
     torch.cuda.synchronize()
@@ -226,7 +147,8 @@ def test_packed_exchange_emulated_ranks(sceneprep_lib, ranks, tree):
     sp.close()
 
 
-@pytest.mark.parametrize("ranks,key_bits,lists", [(2, 32, 3), (3, 6, 3), (4, 20, 3), (7, 3, 3), (8, 32, 3), (16, 10, 3), (8, 12, 40), (5, 4, 97)])
+@pytest.mark.parametrize("ranks,key_bits,lists", [(2, 32, 3), (3, 6, 3), (4, 20, 3), (7, 3, 3), (8, 32, 3), (16, 10, 3), (8, 12, 40), (5, 4, 97),
+                                                   (32, 10, 128)])
 def test_merge_tree_synthetic_runs(sceneprep_lib, ranks, key_bits, lists):
     """The merge-path tree on hand-made blocks: runs of very different lengths (some empty, some spanning many 2048-element
     tiles), few distinct keys (ties decide by rank, then by position in the run) or 32-bit keys. Every rank's slice has to
@@ -235,8 +157,9 @@ def test_merge_tree_synthetic_runs(sceneprep_lib, ranks, key_bits, lists):
     from garden_b200.binding import load_library
     lib = load_library()
     rng = np.random.default_rng(1000 * ranks + key_bits + lists)
-    # (many lists: the (list, pair) job table spans several warp-scan rounds; some lists are empty on every rank)
-    lengths = rng.integers(0, 60000 if lists <= 3 else 5000, size=(ranks, lists))
+    # (many lists: the (list, pair) job table spans several warp-scan rounds; some lists are empty on every rank. 128 lists
+    # at 32 ranks, the largest layout at the largest rank count, fill all 2048 jobs of level 1 with short runs)
+    lengths = rng.integers(0, 60000 if lists <= 3 else 5000 if lists <= 100 else 600, size=(ranks, lists))
     lengths[rng.integers(0, ranks), 0] = 0            # an empty run
     lengths[:, 2] = rng.integers(0, 40, size=ranks)   # a list shorter than one tile
     if ranks >= 3:
@@ -288,3 +211,18 @@ def test_merge_tree_synthetic_runs(sceneprep_lib, ranks, key_bits, lists):
             assert not covered[o + start:o + start + length].any()
             covered[o + start:o + start + length] = True
     assert covered.all()
+
+
+def test_merge_tree_refuses_what_it_cannot_index(sceneprep_lib):
+    """gsp_merge_gathered_packed_tree refuses (GSP_ERR_INVALID, before anything is launched) gathered blocks that reach 2^32
+    words, which its 32-bit element indices cannot address, and more (list, pair of runs) jobs than its table holds. The
+    buffers are tiny placeholders: a refused call reads none of them."""
+    import torch
+    from garden_b200.binding import GSP_ERR_INVALID, load_library
+    lib = load_library()
+    d = torch.zeros(64, dtype=torch.int32, device="cuda").data_ptr()
+    cap = (1 << 30) - 128  # (256 + 2 * cap) * 2 ranks = 2^32 words
+    assert (256 + 2 * cap) * 2 == 1 << 32
+    assert lib.gsp_merge_gathered_packed_tree(0, 2, 0, 3, cap, d, d, d, d, d, d, 16, d) == GSP_ERR_INVALID
+    assert lib.gsp_merge_gathered_packed_tree(0, 32, 0, 129, 16, d, d, d, d, d, d, 16, d) == GSP_ERR_INVALID  # 129 * 16 jobs
+    torch.cuda.synchronize()

@@ -1,9 +1,9 @@
 #!/usr/bin/env python
-"""Single-GPU timing of the exchange's merge (gsp_merge_gathered_packed[_tree]) with the ranks emulated: `ranks` blocks of
+"""Single-GPU timing of the exchange's merge (gsp_merge_gathered_packed_tree) with the ranks emulated: `ranks` blocks of
 sorted runs laid out as the collective leaves them, merged as rank `me`. Runs are `ranks` times longer than a real
 all-to-all sub-block, so that the slice this rank merges has the size it has in a real frame (--slice elements).
 
-  python tools/bench_merge_tree.py --ranks 8 --slice 4400000 [--lists 5] [--reps 50] [--slice-merge]
+  python tools/bench_merge_tree.py --ranks 8 --slice 4400000 [--lists 5] [--reps 50] [--check]
 """
 import argparse
 import json
@@ -23,7 +23,6 @@ def main():
     ap.add_argument("--slice", type=int, default=4_400_000)
     ap.add_argument("--lists", type=int, default=5)
     ap.add_argument("--reps", type=int, default=50)
-    ap.add_argument("--slice-merge", action="store_true", help="time round 1's kMergeSlice instead of the tree")
     ap.add_argument("--check", action="store_true")
     a = ap.parse_args()
     lib = load_library()
@@ -57,12 +56,8 @@ def main():
     me = ranks // 2
 
     def once():
-        if a.slice_merge:
-            rc = lib.gsp_merge_gathered_packed(0, ranks, me, lists, cap, gathered.data_ptr(), plan.data_ptr(), sinfo.data_ptr(),
-                                               out_k.data_ptr(), out_p.data_ptr(), out_r.data_ptr(), total)
-        else:
-            rc = lib.gsp_merge_gathered_packed_tree(0, ranks, me, lists, cap, gathered.data_ptr(), plan.data_ptr(), sinfo.data_ptr(),
-                                                    out_k.data_ptr(), out_p.data_ptr(), out_r.data_ptr(), total, scratch.data_ptr())
+        rc = lib.gsp_merge_gathered_packed_tree(0, ranks, me, lists, cap, gathered.data_ptr(), plan.data_ptr(), sinfo.data_ptr(),
+                                                out_k.data_ptr(), out_p.data_ptr(), out_r.data_ptr(), total, scratch.data_ptr())
         assert rc == 0
     torch.cuda.set_stream(torch.cuda.default_stream())
     for _ in range(5):
@@ -77,7 +72,7 @@ def main():
     ms = e0.elapsed_time(e1) / a.reps
     info = sinfo.cpu().numpy().reshape(lists, 2)
     merged = int(info[:, 1].sum())
-    res = {"ranks": ranks, "lists": lists, "merged_elements": merged, "ms": ms, "kind": "slice" if a.slice_merge else "tree",
+    res = {"ranks": ranks, "lists": lists, "merged_elements": merged, "ms": ms,
            "GBps_per_level_equiv": merged * 18 / ms / 1e6}
     if a.check:
         offs = np.concatenate([[0], np.cumsum(np.array(per_run) * ranks)[:-1]])

@@ -14,7 +14,7 @@ ROOT = Path(__file__).resolve().parent.parent
 LIB = ROOT / "garden_b200" / "libgarden_sceneprep.so"
 OUT = Path(sys.argv[1]) if len(sys.argv) > 1 else ROOT / "profiles" / "r2_sass_hot_kernels.txt"
 HOT = ["kPrepassILj5E", "kCompactSurvivorsILb0E", "kCullILj5ELb0E", "kCullILj5ELb1E", "kClassifyILj5E", "kScanChunks", "kScatter",
-       "kSortPassILb0E", "kEmit", "kTreePartitionILb1E", "kMergeTreeILb1E", "kMergeTreeILb0E", "kPackByDestination", "kSplitRuns",
+       "kSortPass", "kEmit", "kTreePartitionILb1E", "kMergeTreeILb1E", "kMergeTreeILb0E", "kPackByDestination", "kSplitRuns",
        "kInstances", "kAnimate"]
 
 sass = subprocess.run(["cuobjdump", "-sass", str(LIB)], capture_output=True, text=True, check=True).stdout
@@ -58,7 +58,7 @@ for want in HOT:
             ex = excerpt(lines, lambda ls, i: all("FFMA2" in x or "FMUL2" in x for x in ls[i:i + 3]), 2, 30)
             out.append("   -- chain-product step (M <- L(parent) * M):")
             out += ["   " + x for x in ex]
-        if "kSortPassILb0E" in name:
+        if "kSortPass" in name:
             ex = excerpt(lines, lambda ls, i: "R2P" in ls[i], 1, 26)
             out.append("   -- digit peers of one key: predicates of the 8 digit bits (R2P), then vote / and-not / and per bit:")
             out += ["   " + x for x in ex]
