@@ -32,6 +32,8 @@ SYMBOLS = {
     "gsp_update_transforms_indexed": (_i32, [_vp, _vp, _u32, _vp, _u32]),
     "gsp_set_pool_count": (_i32, [_vp, _u32]),
     "gsp_set_mesh_pool": (_i32, [_vp, _u32, _u32, _u32, _vp, _u32, _u32, _u32, _vp]),
+    "gsp_update_mesh_pool": (_i32, [_vp, _u32, _vp, _u32, _u32, _u32, _u32, _vp]),
+    "gsp_update_mesh_pool_indexed": (_i32, [_vp, _u32, _vp, _u32, _vp, _u32, _u32, _vp]),
     "gsp_set_pool_view_mask": (_i32, [_vp, _u32, _u32]),
     "gsp_set_views": (_i32, [_vp, _u32, _vp, _vp]),
     "gsp_run": (_i32, [_vp]),
@@ -195,6 +197,19 @@ class ScenePrep:
             assert ready_counts.size >= occupancy
         self._check(self.lib.gsp_set_mesh_pool(self.h, pool, render_type, 1 if draw_ready else 0, _ptr(aos), stride,
                                                occupancy, count, _ptr(ready_counts)))
+
+    def update_mesh_pool(self, pool: int, aos, stride: int, first: int, count: int, component_count: int,
+                         ready_counts=None):
+        """Restages slots [first, first + count) of a pool set by set_mesh_pool; aos / ready_counts are the pool bases
+        (numpy arrays or raw pointers, host or device)."""
+        self._check(self.lib.gsp_update_mesh_pool(self.h, pool, _ptr(aos), stride, first, count, component_count,
+                                                  _ptr(ready_counts)))
+
+    def update_mesh_pool_indexed(self, pool: int, aos, stride: int, slots, component_count: int, ready_counts=None):
+        """Same for a scattered set of slots (any order, duplicates allowed); aos / ready_counts are host memory."""
+        slots = np.ascontiguousarray(slots, dtype=np.uint32)
+        self._check(self.lib.gsp_update_mesh_pool_indexed(self.h, pool, _ptr(aos), stride, slots.ctypes.data, slots.size,
+                                                          component_count, _ptr(ready_counts)))
 
     def set_pool_view_mask(self, pool: int, view_mask: int):
         """bit v = isDrawReady(views[v].shadowPass) of the pool's mesh system (mesh.cpp:426,482)."""

@@ -26,7 +26,7 @@ static std::string gCreateError;
 	} while (0)
 
 extern "C" { static int fetchWait(Context& c); }
-template<class F> static void parallelFor(uint32_t n, F fn);
+template<class F> static void parallelFor(uint32_t n, F fn, uint32_t minParallel = 1u << 18);
 
 static int fail(Context& c, int code, const char* message)
 {
@@ -181,8 +181,10 @@ int gsp_set_stream(gsp_context* ctx, void* cudaStream)
 //  * pinned / registered host memory (cudaMallocHost, cudaHostRegister, gsp_pin_host): read in place over PCIe by the
 //    staging kernel ("zero copy") — no intermediate device buffer, the re-layout overlaps the transfer;
 //  * device memory: read in place;
-//  * pageable host memory: copied into a device scratch buffer first (cudaMemcpyAsync stages it through the driver).
-static int resolveSource(Context& c, const void* aos, size_t bytes, const void** src)
+//  * pageable host memory: copied into a device scratch buffer first (cudaMemcpyAsync stages it through the driver), at
+//    `scratchOffset`. A call with two sources puts the second behind the first and reserves room for both BEFORE the first
+//    resolveSource: growing the scratch here would free the buffer the first source's pointer points into.
+static int resolveSource(Context& c, const void* aos, size_t bytes, const void** src, size_t scratchOffset = 0)
 {
 	cudaPointerAttributes attr = {};
 	cudaError_t err = cudaPointerGetAttributes(&attr, aos);
@@ -204,10 +206,68 @@ static int resolveSource(Context& c, const void* aos, size_t bytes, const void**
 	}
 	size_t cap = c.dAosScratchCap;
 	uint8_t* ptr = (uint8_t*)c.dAosScratch;
+	GSP_CUDA(ensureDevice(ptr, cap, scratchOffset + bytes, false, c.stream));
+	c.dAosScratch = ptr; c.dAosScratchCap = cap;
+	GSP_CUDA(cudaMemcpyAsync((uint8_t*)c.dAosScratch + scratchOffset, aos, bytes, cudaMemcpyHostToDevice, c.stream));
+	*src = (uint8_t*)c.dAosScratch + scratchOffset;
+	return GSP_OK;
+}
+
+static bool isDevicePointer(const void* p)
+{
+	cudaPointerAttributes attr = {};
+	if (cudaPointerGetAttributes(&attr, p) != cudaSuccess)
+	{
+		cudaGetLastError();
+		return false;
+	}
+	return attr.type == cudaMemoryTypeDevice;
+}
+
+// A scattered dirty set as ONE upload: slots[count], then the components aos[slots[i]] back to back, then (ready != nullptr)
+// the bytes ready[slots[i]], packed in pinned memory and copied into the device scratch buffer. Host memory only.
+struct Gathered
+{
+	const uint32_t* slots;
+	const uint8_t* aos;
+	const uint8_t* ready;
+};
+static int uploadGathered(Context& c, const void* aos, uint32_t stride, const uint32_t* slots, uint32_t count,
+	const uint8_t* ready, Gathered* out)
+{
+	const size_t listBytes = ((size_t)count * sizeof(uint32_t) + 15) & ~(size_t)15;
+	const size_t aosBytes = (size_t)count * stride;
+	const size_t bytes = listBytes + aosBytes + (ready ? count : 0);
+	if (c.hGatherCap < bytes)
+	{
+		GSP_CUDA(cudaStreamSynchronize(c.stream));
+		cudaFreeHost(c.hGather); c.hGather = nullptr; c.hGatherCap = 0;
+		const size_t cap = bytes + bytes / 2;
+		GSP_CUDA(cudaMallocHost((void**)&c.hGather, cap));
+		c.hGatherCap = cap;
+	}
+	memcpy(c.hGather, slots, (size_t)count * sizeof(uint32_t));
+	const uint8_t* src = (const uint8_t*)aos;
+	uint8_t* packed = c.hGather + listBytes;
+	uint8_t* packedReady = packed + aosBytes;
+	parallelFor(count, [=](uint32_t first, uint32_t last)
+	{
+		for (uint32_t i = first; i < last; i++)
+		{
+			memcpy(packed + (size_t)i * stride, src + (size_t)slots[i] * stride, stride);
+			if (ready)
+				packedReady[i] = ready[slots[i]];
+		}
+	}, 1u << 14); // (each row is a cache miss at a scattered address: workers pay off far below the default threshold)
+	size_t cap = c.dAosScratchCap;
+	uint8_t* ptr = (uint8_t*)c.dAosScratch;
 	GSP_CUDA(ensureDevice(ptr, cap, bytes, false, c.stream));
 	c.dAosScratch = ptr; c.dAosScratchCap = cap;
-	GSP_CUDA(cudaMemcpyAsync(c.dAosScratch, aos, bytes, cudaMemcpyHostToDevice, c.stream));
-	*src = c.dAosScratch;
+	GSP_CUDA(cudaMemcpyAsync(c.dAosScratch, c.hGather, bytes, cudaMemcpyHostToDevice, c.stream));
+	const uint8_t* d = (const uint8_t*)c.dAosScratch;
+	out->slots = (const uint32_t*)d;
+	out->aos = d + listBytes;
+	out->ready = ready ? d + listBytes + aosBytes : nullptr;
 	return GSP_OK;
 }
 
@@ -348,31 +408,10 @@ int gsp_update_transforms_indexed(gsp_context* ctx, const void* aos, uint32_t st
 		if (slots[i] >= c.tf.occupancy)
 			return fail(c, GSP_ERR_INVALID, "gsp_update_transforms_indexed: slot index out of range");
 	GSP_CUDA(cudaSetDevice(c.device));
-	// the dirty components are packed back to back behind their slot list in pinned memory and travel as ONE copy
-	const size_t listBytes = ((size_t)count * sizeof(uint32_t) + 15) & ~(size_t)15;
-	const size_t bytes = listBytes + (size_t)count * stride;
-	if (c.hGatherCap < bytes)
-	{
-		GSP_CUDA(cudaStreamSynchronize(c.stream));
-		cudaFreeHost(c.hGather); c.hGather = nullptr; c.hGatherCap = 0;
-		const size_t cap = bytes + bytes / 2;
-		GSP_CUDA(cudaMallocHost((void**)&c.hGather, cap));
-		c.hGatherCap = cap;
-	}
-	memcpy(c.hGather, slots, (size_t)count * sizeof(uint32_t));
-	const uint8_t* src = (const uint8_t*)aos;
-	uint8_t* packed = c.hGather + listBytes;
-	parallelFor(count, [=](uint32_t first, uint32_t last)
-	{
-		for (uint32_t i = first; i < last; i++)
-			memcpy(packed + (size_t)i * stride, src + (size_t)slots[i] * stride, stride);
-	});
-	size_t cap = c.dAosScratchCap;
-	uint8_t* ptr = (uint8_t*)c.dAosScratch;
-	GSP_CUDA(ensureDevice(ptr, cap, bytes, false, c.stream));
-	c.dAosScratch = ptr; c.dAosScratchCap = cap;
-	GSP_CUDA(cudaMemcpyAsync(c.dAosScratch, c.hGather, bytes, cudaMemcpyHostToDevice, c.stream));
-	launchStageTransforms(c, (const uint8_t*)c.dAosScratch + listBytes, stride, 0, count, false, nullptr, (const uint32_t*)c.dAosScratch);
+	Gathered g;
+	int rc = uploadGathered(c, aos, stride, slots, count, nullptr, &g);
+	if (rc) return rc;
+	launchStageTransforms(c, g.aos, stride, 0, count, false, nullptr, g.slots);
 	c.chainDirty = true;
 	GSP_CUDA(cudaStreamSynchronize(c.stream)); // the pinned gather buffer is free again
 	GSP_CUDA(cudaGetLastError());
@@ -456,12 +495,120 @@ int gsp_set_mesh_pool(gsp_context* ctx, uint32_t pool, uint32_t renderType, uint
 	const void* src = nullptr;
 	int rc = resolveSource(c, aos, (size_t)stride * occupancy, &src);
 	if (rc) return rc;
-	launchStagePool(c, pool, src, stride, occupancy);
+	launchStagePool(c, pool, src, stride, 0, occupancy);
 	if (readyCounts)
 		GSP_CUDA(cudaMemcpyAsync(p.ready, readyCounts, occupancy, cudaMemcpyHostToDevice, c.stream));
 	GSP_CUDA(cudaStreamSynchronize(c.stream));
 	GSP_CUDA(cudaGetLastError());
 	return GSP_OK;
+}
+
+// Arguments every gsp_update_mesh_pool* call checks before it changes anything.
+static int checkMeshUpdate(Context& c, uint32_t pool, uint32_t stride, bool pointers, const uint8_t* readyCounts, const char* who)
+{
+	if (pool >= (uint32_t)kMaxPools)
+		return fail(c, GSP_ERR_INVALID, (std::string(who) + ": bad pool index").c_str());
+	auto& p = c.pools[pool];
+	if (!p.set)
+		return fail(c, GSP_ERR_STATE, (std::string(who) + ": the pool has not been set (gsp_set_mesh_pool)").c_str());
+	if (stride != p.stride || !pointers || (readyCounts != nullptr) != p.hasReady)
+		return fail(c, GSP_ERR_INVALID, (std::string(who) + ": null pointer, a stride other than the staged one, or ready "
+			"counts given for a pool staged without them (or the reverse)").c_str());
+	return GSP_OK;
+}
+
+// The listed slots were restaged by kStagePool (dSlotMap, else first + i). Links them incrementally instead of marking the link
+// dirty: the next frame then launches what a frame after no change launches. Ends in a stream synchronisation.
+static int relinkMeshSlots(Context& c, uint32_t pool, const uint32_t* dSlotMap, uint32_t first, uint32_t count,
+	uint32_t componentCount)
+{
+	auto& p = c.pools[pool];
+	// a pending full link / chain pass of the next frame covers these slots (and needs the current rho, tslot)
+	const bool link = !c.linkDirty, walk = link && !c.chainDirty;
+	uint32_t* dGrew = c.dCounters + kCtrError + 1;
+	uint32_t* hGrew = c.hCounters + kCtrCount;
+	if (link)
+	{
+		GSP_CUDA(cudaMemsetAsync(dGrew, 0, sizeof(uint32_t), c.stream));
+		launchLinkSlots(c, pool, dSlotMap, first, count, walk, dGrew);
+		GSP_CUDA(cudaMemcpyAsync(hGrew, dGrew, sizeof(uint32_t), cudaMemcpyDeviceToHost, c.stream));
+	}
+	GSP_CUDA(cudaStreamSynchronize(c.stream)); // the scratch buffer and the caller's memory are free again
+	GSP_CUDA(cudaGetLastError());
+	if (walk && *hGrew)
+	{
+		launchChainRecords(c);
+		GSP_CUDA(cudaStreamSynchronize(c.stream));
+		GSP_CUDA(cudaGetLastError());
+	}
+	if ((p.count == 0) != (componentCount == 0))
+		c.layoutDirty = true;
+	p.count = componentCount;
+	p.visibleValid = false;
+	c.resultsValid = false; c.frameEnqueued = false;
+	return GSP_OK;
+}
+
+int gsp_update_mesh_pool(gsp_context* ctx, uint32_t pool, const void* aos, uint32_t stride, uint32_t first, uint32_t count,
+	uint32_t componentCount, const uint8_t* readyCounts)
+{
+	if (!ctx)
+		return GSP_ERR_INVALID;
+	Context& c = ctx->c;
+	int rc = checkMeshUpdate(c, pool, stride, aos || !count, readyCounts, "gsp_update_mesh_pool");
+	if (rc) return rc;
+	auto& p = c.pools[pool];
+	if ((uint64_t)first + count > p.occupancy)
+		return fail(c, GSP_ERR_INVALID, "gsp_update_mesh_pool: range past the staged occupancy (gsp_set_mesh_pool grows it)");
+	if (count == 0)
+		return GSP_OK;
+	GSP_CUDA(cudaSetDevice(c.device));
+	// `aos` / `readyCounts` are the pool bases; only the range is read, each from where it lives (resolveSource)
+	const size_t aosBytes = (size_t)stride * count;
+	const size_t readyOffset = (aosBytes + 15) & ~(size_t)15;
+	{
+		// room for both sources before either is resolved (see resolveSource)
+		size_t cap = c.dAosScratchCap;
+		uint8_t* ptr = (uint8_t*)c.dAosScratch;
+		GSP_CUDA(ensureDevice(ptr, cap, readyCounts ? readyOffset + count : aosBytes, false, c.stream));
+		c.dAosScratch = ptr; c.dAosScratchCap = cap;
+	}
+	const void* src = nullptr;
+	const void* readySrc = nullptr;
+	rc = resolveSource(c, (const uint8_t*)aos + (size_t)first * stride, aosBytes, &src);
+	if (rc) return rc;
+	if (readyCounts)
+	{
+		rc = resolveSource(c, readyCounts + first, count, &readySrc, readyOffset);
+		if (rc) return rc;
+	}
+	launchStagePool(c, pool, src, stride, first, count, nullptr, (const uint8_t*)readySrc);
+	return relinkMeshSlots(c, pool, nullptr, first, count, componentCount);
+}
+
+int gsp_update_mesh_pool_indexed(gsp_context* ctx, uint32_t pool, const void* aos, uint32_t stride, const uint32_t* slots,
+	uint32_t count, uint32_t componentCount, const uint8_t* readyCounts)
+{
+	if (!ctx)
+		return GSP_ERR_INVALID;
+	Context& c = ctx->c;
+	int rc = checkMeshUpdate(c, pool, stride, (aos && slots) || !count, readyCounts, "gsp_update_mesh_pool_indexed");
+	if (rc) return rc;
+	if (count == 0)
+		return GSP_OK;
+	GSP_CUDA(cudaSetDevice(c.device));
+	// the library reads all three on the host while it packs them
+	if (isDevicePointer(aos) || isDevicePointer(slots) || (readyCounts && isDevicePointer(readyCounts)))
+		return fail(c, GSP_ERR_INVALID, "gsp_update_mesh_pool_indexed: the components, slots and ready counts must be host memory");
+	auto& p = c.pools[pool];
+	for (uint32_t i = 0; i < count; i++)
+		if (slots[i] >= p.occupancy)
+			return fail(c, GSP_ERR_INVALID, "gsp_update_mesh_pool_indexed: slot index past the staged occupancy");
+	Gathered g;
+	rc = uploadGathered(c, aos, stride, slots, count, readyCounts, &g);
+	if (rc) return rc;
+	launchStagePool(c, pool, g.aos, stride, 0, count, g.slots, g.ready);
+	return relinkMeshSlots(c, pool, g.slots, 0, count, componentCount);
 }
 
 int gsp_set_pool_view_mask(gsp_context* ctx, uint32_t pool, uint32_t viewMask)
@@ -1430,9 +1577,9 @@ private:
 } // namespace
 
 template<class F>
-static void parallelFor(uint32_t n, F fn)
+static void parallelFor(uint32_t n, F fn, uint32_t minParallel)
 {
-	if (n < (1u << 18) || HostWorkers::get().size() == 1)
+	if (n < minParallel || HostWorkers::get().size() == 1)
 	{
 		fn(0u, n);
 		return;

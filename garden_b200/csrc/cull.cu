@@ -202,29 +202,78 @@ struct ChainArgs
 	float4* __restrict__ record;
 	uint32_t count;
 };
+// Walks the parent chain of transform t (D, S above) and returns its root; `beyond`: the chain is longer than the walk allows.
+__device__ __forceinline__ uint32_t chainWalk(const float2* __restrict__ bound, const uint32_t* __restrict__ parent, uint32_t t,
+	float& D, float& S, bool& beyond)
+{
+	const float2 own = bound[t];
+	float tauPrev = own.y;
+	D = 0.0f; S = own.x;
+	uint32_t root = t, p = parent[t], n = 0;
+	while (p != kNone && n < kPreMaxWalk)
+	{
+		const float2 b = bound[p];
+		const float d = b.x * (tauPrev + D), s = b.x * S;
+		D = fmaf(d, 0x1p-8f, d); S = fmaf(s, 0x1p-8f, s);
+		tauPrev = b.y; root = p; p = parent[p]; n++;
+	}
+	beyond = p != kNone;
+	return root;
+}
+// u = D + S * rho, the reach of a mesh of box radius rho on the transform from its root's position
+__device__ __forceinline__ float chainReach(float D, float S, float rho, bool beyond)
+{
+	float u = rho == 0.0f ? D : fmaf(S, rho, D); // (0 * inf would poison a transform that carries no mesh)
+	if (beyond) // longer than the walk allows (or cyclic): nothing of this hierarchy is ever culled by the prepass
+		u = __int_as_float(0x7f800000);
+	return u;
+}
 __global__ void __launch_bounds__(256) kChainBounds(const __grid_constant__ ChainArgs A)
 {
 	const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
 	if (t >= A.count)
 		return;
-	const float2 own = A.bound[t];
-	float D = 0.0f, S = own.x, tauPrev = own.y;
-	uint32_t root = t, p = A.parent[t], n = 0;
-	while (p != kNone && n < kPreMaxWalk)
-	{
-		const float2 b = A.bound[p];
-		const float d = b.x * (tauPrev + D), s = b.x * S;
-		D = fmaf(d, 0x1p-8f, d); S = fmaf(s, 0x1p-8f, s);
-		tauPrev = b.y; root = p; p = A.parent[p]; n++;
-	}
-	const float rho = __uint_as_float(A.rho[t]);
-	float u = rho == 0.0f ? D : fmaf(S, rho, D); // (0 * inf would poison a transform that carries no mesh)
-	if (p != kNone) // longer than the walk allows (or cyclic): nothing of this hierarchy is ever culled by the prepass
-		u = __int_as_float(0x7f800000);
+	float D, S;
+	bool beyond;
+	const uint32_t root = chainWalk(A.bound, A.parent, t, D, S, beyond);
+	const float u = chainReach(D, S, __uint_as_float(A.rho[t]), beyond);
 	A.chainRoot[t] = root;
 	// u >= +0, +inf or NaN: the bit patterns order like unsigned integers (NaN on top)
 	if ((A.flags[t] & kTfLive) && (A.flags[root] & kTfLive))
 		atomicMax(&A.rootW[root], __float_as_uint(u));
+}
+// Incremental link of the pool slots that gsp_update_mesh_pool[_indexed] restaged (slotMap[i], else first + i): the slot's
+// transform slot, and its box radius folded into rho as kLinkPool does. rho only grows here: a smaller or moved box keeps the
+// larger sphere, still conservative, until the next full link. *grew = 1 when some rho grew; with `walk` (the chain bounds
+// are current) such a transform's chain is walked as kChainBounds walks it and its reach folded into rootW[root]. Each thread
+// folds its own radius: the largest one that raised rho reaches rootW, so rootW covers the final rho. The records then need
+// kChainRecords.
+__global__ void __launch_bounds__(256) kLinkSlots(const uint32_t* __restrict__ slotMap, uint32_t first, uint32_t count,
+	const uint32_t* __restrict__ entity, const uint32_t* __restrict__ entityToSlot, uint32_t entityCap,
+	uint32_t* __restrict__ tslot, const float* __restrict__ radius, uint32_t* rho, int walk, const float2* __restrict__ bound,
+	const uint32_t* __restrict__ parent, const uint16_t* __restrict__ tFlags, uint32_t* rootW, uint32_t* __restrict__ grew)
+{
+	const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+	if (i >= count)
+		return;
+	const uint32_t slot = slotMap ? slotMap[i] : first + i;
+	const uint32_t e = entity[slot];
+	const uint32_t s = (e && e < entityCap) ? entityToSlot[e] : 0;
+	tslot[slot] = s ? s - 1 : kNone;
+	if (!s)
+		return;
+	const uint32_t t = s - 1, r = __float_as_uint(radius[slot]);
+	if (atomicMax(&rho[t], r) >= r)
+		return;
+	*grew = 1;
+	if (!walk)
+		return;
+	float D, S;
+	bool beyond;
+	const uint32_t root = chainWalk(bound, parent, t, D, S, beyond);
+	const float u = chainReach(D, S, __uint_as_float(r), beyond);
+	if ((tFlags[t] & kTfLive) && (tFlags[root] & kTfLive))
+		atomicMax(&rootW[root], __float_as_uint(u));
 }
 __global__ void __launch_bounds__(256) kChainRecords(const __grid_constant__ ChainArgs A)
 {
@@ -1465,19 +1514,48 @@ static void prepareBoxGroup(CullParams& P)
 	P.boxSlack = (float)(slack * 1.0001);
 }
 
+static ChainArgs chainArgs(const TransformsDev& t)
+{
+	ChainArgs A;
+	A.bound = t.bound; A.parent = t.parent; A.flags = t.flags; A.posSx = t.posSx; A.rho = t.rho;
+	A.chainRoot = t.chainRoot; A.rootW = t.rootW; A.record = t.record; A.count = t.occupancy;
+	return A;
+}
+
 // Prepass spheres of every transform: once per change of transforms, pools or active flags (after launchLink: needs rho)
 uint32_t launchChainBounds(Context& c)
 {
 	auto& t = c.tf;
 	if (t.occupancy == 0)
 		return 0;
-	ChainArgs A;
-	A.bound = t.bound; A.parent = t.parent; A.flags = t.flags; A.posSx = t.posSx; A.rho = t.rho;
-	A.chainRoot = t.chainRoot; A.rootW = t.rootW; A.record = t.record; A.count = t.occupancy;
+	const ChainArgs A = chainArgs(t);
 	cudaMemsetAsync(t.rootW, 0, (size_t)t.occupancy * sizeof(uint32_t), c.stream);
 	kChainBounds<<<(t.occupancy + 255) / 256, 256, 0, c.stream>>>(A);
 	kChainRecords<<<(t.occupancy + 255) / 256, 256, 0, c.stream>>>(A);
 	return 2;
+}
+
+// The records alone, from rho and rootW as they stand (after kLinkSlots grew some of them)
+uint32_t launchChainRecords(Context& c)
+{
+	auto& t = c.tf;
+	if (t.occupancy == 0)
+		return 0;
+	kChainRecords<<<(t.occupancy + 255) / 256, 256, 0, c.stream>>>(chainArgs(t));
+	return 1;
+}
+
+// *dGrew (zeroed by the caller) = 1 when some rho grew. `walk` needs rootW and chainRoot of the current transforms.
+uint32_t launchLinkSlots(Context& c, uint32_t pool, const uint32_t* dSlotMap, uint32_t first, uint32_t count, bool walk,
+	uint32_t* dGrew)
+{
+	auto& t = c.tf;
+	auto& p = c.pools[pool];
+	if (count == 0)
+		return 0;
+	kLinkSlots<<<(count + 255) / 256, 256, 0, c.stream>>>(dSlotMap, first, count, p.entity, t.entityToSlot, t.entityCap,
+		p.tslot, p.radius, t.rho, walk ? 1 : 0, t.bound, t.parent, t.flags, t.rootW, dGrew);
+	return 1;
 }
 
 static void setKernelAttributes(Context& c)

@@ -262,9 +262,13 @@ uint32_t launchStageTransforms(Context& c, const void* dAos, uint32_t stride, ui
 	uint32_t* dMaxEntity, const uint32_t* dSlotMap = nullptr);
 uint32_t launchBuildHierarchy(Context& c, uint32_t* dDeep);
 uint32_t launchFindCycles(Context& c, uint32_t* dCyclic);
-uint32_t launchStagePool(Context& c, uint32_t pool, const void* dAos, uint32_t stride, uint32_t occupancy);
+uint32_t launchStagePool(Context& c, uint32_t pool, const void* dAos, uint32_t stride, uint32_t first, uint32_t count,
+	const uint32_t* dSlotMap = nullptr, const uint8_t* dReady = nullptr);
 uint32_t launchLink(Context& c);
 uint32_t launchChainBounds(Context& c);
+uint32_t launchLinkSlots(Context& c, uint32_t pool, const uint32_t* dSlotMap, uint32_t first, uint32_t count, bool walk,
+	uint32_t* dGrew);
+uint32_t launchChainRecords(Context& c);
 uint32_t launchSplitWorld(Context& c, cudaEvent_t before, cudaEvent_t after);
 uint32_t launchCull(Context& c, uint32_t pool, cudaEvent_t afterPrepass, cudaEvent_t afterCull, cudaEvent_t afterScatter);
 uint32_t launchSort(Context& c, cudaEvent_t afterHistogram);

@@ -185,10 +185,12 @@ __global__ void __launch_bounds__(256) kJumpParents(uint32_t count, uint32_t* up
 }
 
 // One block per tile of mesh-component slots: AABB, owner entity, the static part of the filter at mesh.cpp:140-147, and the
-// isVisible byte the host currently holds (for the changed-slots-only write-back).
-__global__ void __launch_bounds__(kStageThreads) kStagePool(const uint8_t* __restrict__ aos, uint32_t stride, uint32_t count,
-	uint32_t tileSlots, float4* __restrict__ aabbA, float2* __restrict__ aabbB, uint32_t* __restrict__ entity,
-	uint8_t* __restrict__ flags, float* __restrict__ radius)
+// isVisible byte the host currently holds (for the changed-slots-only write-back). `readySrc` (nullable): the ready counts of
+// the staged components, in the same order.
+__global__ void __launch_bounds__(kStageThreads) kStagePool(const uint8_t* __restrict__ aos, uint32_t stride, uint32_t first,
+	uint32_t count, uint32_t tileSlots, const uint32_t* __restrict__ slotMap, const uint8_t* __restrict__ readySrc,
+	float4* __restrict__ aabbA, float2* __restrict__ aabbB, uint32_t* __restrict__ entity, uint8_t* __restrict__ flags,
+	float* __restrict__ radius, uint8_t* __restrict__ ready)
 {
 	extern __shared__ __align__(16) uint8_t sTile[];
 	const uint32_t tileFirst = blockIdx.x * tileSlots;
@@ -196,7 +198,8 @@ __global__ void __launch_bounds__(kStageThreads) kStagePool(const uint8_t* __res
 	loadTile(sTile, aos + (size_t)tileFirst * stride, n * stride);
 	for (uint32_t j = threadIdx.x; j < n; j += kStageThreads)
 	{
-		const uint32_t i = tileFirst + j;
+		// slotMap: the j-th staged component belongs to slot slotMap[j] (scattered dirty set), else to first + j (a range)
+		const uint32_t i = slotMap ? slotMap[tileFirst + j] : first + tileFirst + j;
 		const uint8_t* m = sTile + (size_t)j * stride;
 		uint32_t e = ldU32(m + kMcEntity);
 		uint32_t w = ldU32(m + 12); // bytes 12..15: reserved2 (u16), isEnabled, isVisible
@@ -214,6 +217,8 @@ __global__ void __launch_bounds__(kStageThreads) kStagePool(const uint8_t* __res
 		if (hostVisible == 1) f |= kMfHostVisible;          // the host byte is a clean `true`
 		else if (hostVisible != 0) f |= kMfHostVisibleOdd;  // neither 0 nor 1: always rewritten
 		flags[i] = f;
+		if (readySrc)
+			ready[i] = readySrc[tileFirst + j];
 	}
 }
 
@@ -316,16 +321,17 @@ uint32_t launchFindCycles(Context& c, uint32_t* dCyclic)
 	return rounds;
 }
 
-uint32_t launchStagePool(Context& c, uint32_t pool, const void* dAos, uint32_t stride, uint32_t occupancy)
+uint32_t launchStagePool(Context& c, uint32_t pool, const void* dAos, uint32_t stride, uint32_t first, uint32_t count,
+	const uint32_t* dSlotMap, const uint8_t* dReady)
 {
-	if (occupancy == 0)
+	if (count == 0)
 		return 0;
 	auto& p = c.pools[pool];
 	size_t smem;
 	const uint32_t tileSlots = tileSlotsFor(stride, smem);
 	cudaFuncSetAttribute(kStagePool, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
-	kStagePool<<<blocksFor(occupancy, tileSlots), kStageThreads, smem, c.stream>>>((const uint8_t*)dAos, stride, occupancy,
-		tileSlots, p.aabbA, p.aabbB, p.entity, p.flags, p.radius);
+	kStagePool<<<blocksFor(count, tileSlots), kStageThreads, smem, c.stream>>>((const uint8_t*)dAos, stride, first, count,
+		tileSlots, dSlotMap, dReady, p.aabbA, p.aabbB, p.entity, p.flags, p.radius, p.ready);
 	return 1;
 }
 

@@ -104,6 +104,28 @@ int gsp_set_pool_count(gsp_context* ctx, uint32_t poolCount);
  * getReadyMeshesAsync override beyond the frustum test (e.g. sprite.cpp:90-97): ready instance count per slot. */
 int gsp_set_mesh_pool(gsp_context* ctx, uint32_t pool, uint32_t renderType, uint32_t drawReady, const void* aos,
 	uint32_t stride, uint32_t occupancy, uint32_t count, const uint8_t* readyCounts);
+/* MeshRenderComponent changes (mesh.hpp:45-55: entity, isEnabled, isVisible, aabb) of slots [first, first + count) of a pool
+ * staged by gsp_set_mesh_pool: a mesh hidden or shown, a box swapped, a sprite that became ready, a component destroyed
+ * (entity = 0) or a freed slot reused by an entity that already has a transform. `aos` and `readyCounts` are the pool /
+ * ready-count bases (same meaning as gsp_set_mesh_pool); only the listed slots are read, from pinned, device or pageable memory
+ * as in gsp_set_transforms. componentCount = LinearPool::getCount() after the change (linear-pool.hpp:729).
+ * Every result afterwards is what a context would give that had staged the same bytes with gsp_set_mesh_pool, but the pool is
+ * not re-uploaded and the next frame does not relink: a grown box widens its hierarchy's prepass sphere in place, a shrunken
+ * or moved box keeps the larger sphere (only a gsp_set_mesh_pool or gsp_set_transforms tightens it again). Like
+ * gsp_set_mesh_pool, the call ends the frame's results (gsp_writeback_visible* are no-ops until the next run), keeps a
+ * gsp_fetch_all_async snapshot unless componentCount changes between zero and non-zero (a new list layout), and takes the
+ * library's copy of the host's isVisible byte of the listed slots from the uploaded bytes.
+ * GSP_ERR_STATE: the pool was never set. GSP_ERR_INVALID: pool >= GSP_MAX_POOLS, a stride other than the staged one, a slot at
+ * or past the staged occupancy (growing it is gsp_set_mesh_pool's), readyCounts given for a pool staged without ready counts
+ * or the reverse, a null pointer with count > 0. A refused call changes nothing. These checks come first: a call that passes
+ * them with count == 0 is a no-op (so a range must still start at or below the occupancy, and the pool must have been set,
+ * as for gsp_update_transforms). */
+int gsp_update_mesh_pool(gsp_context* ctx, uint32_t pool, const void* aos, uint32_t stride, uint32_t first, uint32_t count,
+	uint32_t componentCount, const uint8_t* readyCounts);
+/* Same for a scattered set: slots[count] (any order, duplicates allowed). `aos`, `slots` and `readyCounts` are host memory
+ * (a device pointer is refused with GSP_ERR_INVALID); the listed components travel packed in one pinned upload. */
+int gsp_update_mesh_pool_indexed(gsp_context* ctx, uint32_t pool, const void* aos, uint32_t stride, const uint32_t* slots,
+	uint32_t count, uint32_t componentCount, const uint8_t* readyCounts);
 /* IMeshRenderSystem::isDrawReady(shadowPass) is asked once per prepareMeshes call, i.e. per VIEW (mesh.cpp:426,482), and
  * systems answer per kind of pass: InstanceRenderSystem checks the base pipeline for shadowPass < 0 and the shadow pipeline
  * otherwise (source/system/render/instance.cpp:61-113; createShadowPipeline() returns {} by default), UiLabelSystem returns
